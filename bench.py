@@ -10,6 +10,11 @@ forward and backward (gradients to every disparity scale and to the poses).
 Metric: warped px-pairs per second (SURVEY.md 8d), whole job over all ranks.
 
 Prints ONE JSON line (rank 0).  See DESIGN.md "Measurement" for every key.
+
+    python bench.py ... --dump-outputs DIR
+
+also writes what the last timed step computed (losses, the gradients of every leaf, the depth planes) as
+DIR/<name>.npy, so that two builds can be compared output for output on identical seeded inputs.
 """
 from __future__ import annotations
 
@@ -23,6 +28,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True   # the benchmark leaves the source tree as it found it (it may be read-only)
 
 import torch  # noqa: E402
 
@@ -46,7 +52,44 @@ def parse():
                     help="skip the full-training-step sub-record (BASELINE.json configs[4])")
     ap.add_argument("--with-pose", action="store_true",
                     help="include the pose assembly (axis-angle/translation -> T, SURVEY 8f-2) in the timed step")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step computed as DIR/<name>.npy (float32, at most 64 MB in all)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.workload in FULL_STEP):
+        ap.error("--dump-outputs covers the fused loss path (--impl ours, a loss workload)")
+    return args
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def collect_outputs(losses, leaves, outputs):
+    """What a caller of loss_step + backward receives from one step: the losses, the gradient of every leaf and
+    the depth planes loss_step stores in ``outputs``; copied to the host as float32 numpy arrays."""
+    def name(k):
+        return "_".join(str(p) for p in k) if isinstance(k, tuple) else str(k)
+
+    arrays = {name(k).replace("/", "_"): v for k, v in losses.items()}
+    arrays.update({"grad_" + name(k): p.grad for k, p in leaves.items()})
+    arrays.update({name(k): v for k, v in outputs.items() if isinstance(k, tuple) and k[0] == "depth"})
+    return {k: v.detach().float().cpu().numpy() for k, v in arrays.items()}
+
+
+def write_outputs(directory, arrays):
+    """Save ``arrays`` as ``directory/<name>.npy``.  Past DUMP_LIMIT_BYTES in all, every array keeps the same share of
+    its elements, picked by a fixed seed (flat indices, ascending), so that two runs keep the same elements."""
+    import numpy as np
+    os.makedirs(directory, exist_ok=True)
+    total = sum(a.nbytes for a in arrays.values())
+    room = DUMP_LIMIT_BYTES - 1024 * len(arrays)          # the .npy headers
+    keep = min(1.0, room / total) if total else 1.0
+    for k, a in sorted(arrays.items()):
+        if keep < 1.0 and a.size > 1:
+            idx = np.sort(np.random.default_rng(0).choice(a.size, max(1, int(a.size * keep)), replace=False))
+            a = a.reshape(-1)[idx]
+        np.save(os.path.join(directory, k + ".npy"), a)
 
 
 # ----------------------------------------------------------------------------------------------
@@ -298,9 +341,10 @@ def run_ours(args):
         # baseline group, exactly like compute_losses does (trainer.py:518-523)
         losses = loss_step(inputs, outputs, opt, plan, noise=None, num_scales=4, timers=timers)
         losses["loss"].backward()
-        return losses["loss"]
+        return losses
 
     # ---- device-resident timing ------------------------------------------------------------
+    torch.manual_seed(4321 + rank)   # the noise drawn inside the steps: the same from run to run
     sampler.mark()                # clock samples count from the warm-up to the end of the e2e loop
     for _ in range(max(3, args.warmup)):
         for p in leaves.values():
@@ -318,11 +362,12 @@ def run_ours(args):
         if not os.environ.get("BBD_BENCH_NO_FLUSH"): flush.zero_()
         timers.clear()
         ev[i][0].record()
-        step()
+        last = step()
         ev[i][1].record()
         kernel_ev.append(timers.get("reproj_fused"))
     barrier()
     wall = time.perf_counter() - wall0
+    dump = collect_outputs(last, leaves, outputs) if args.dump_outputs and rank == 0 else None
     launches = be.launches
     step_ms = sum(a.elapsed_time(b) for a, b in ev) / args.steps
     kern_ms = sum(a.elapsed_time(b) for a, b in kernel_ev if a is not None) / max(1, len(kernel_ev))
@@ -350,12 +395,15 @@ def run_ours(args):
             side = torch.cuda.Stream()
             side.wait_stream(torch.cuda.current_stream())
             with torch.cuda.stream(side):
-                if args.with_pose:
-                    # fresh leaves: their gradient-accumulation nodes must not belong to the legacy default stream
-                    # the eager loop above ran on (autograd would make that stream wait for the capturing one)
-                    for k in list(pose_params):
-                        pose_params[k] = pose_params[k].detach().clone().requires_grad_(True)
-                        leaves[k] = pose_params[k]
+                # fresh leaves: their gradient-accumulation nodes must not belong to the legacy default stream
+                # the eager loop above ran on (autograd would make that stream wait for the capturing one, which
+                # invalidates the capture)
+                for k in list(leaves):
+                    leaves[k] = leaves[k].detach().clone().requires_grad_(True)
+                    if k in pose_params:
+                        pose_params[k] = leaves[k]
+                    else:                                    # ("disp", s) and ("cam_T_cam", 0, f) are outputs entries
+                        outputs[k] = leaves[k]
                 for _ in range(3):
                     for p in leaves.values():
                         p.grad = None
@@ -365,7 +413,7 @@ def run_ours(args):
                 p.grad = None
             g = torch.cuda.CUDAGraph()
             with torch.cuda.graph(g):
-                step()
+                static_losses = step()
             gev = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(args.steps)]
             barrier()
             for i in range(args.steps):
@@ -375,12 +423,16 @@ def run_ours(args):
                 gev[i][1].record()
             barrier()
             graph_ms = sum(a.elapsed_time(b) for a, b in gev) / args.steps
+            if dump is not None:    # the replayed step is the headline: its last replay is what gets written
+                dump = collect_outputs(static_losses, leaves, outputs)
         except Exception as exc:  # noqa: BLE001
             graph_ms = None
             print(f"graph capture failed: {type(exc).__name__}: {exc}", file=sys.stderr)
             if os.environ.get("BBD_BENCH_DEBUG"):
                 import traceback
                 traceback.print_exc()
+    if dump is not None:
+        write_outputs(args.dump_outputs, dump)
 
     # ---- end to end: pinned host batch -> H2D -> fused loss fwd+bwd -> D2H loss ---------------
     # Every step uploads its whole batch (images, pyramid, K, stereo_T, disparities, camera motions)
@@ -471,7 +523,7 @@ def run_ours(args):
 
             e2e_run(3)
             barrier()
-            n_e2e = max(10, min(args.steps, 50))
+            n_e2e = args.steps
             runs = []
             for _ in range(3):                       # three timed loops, the median is reported
                 if not os.environ.get("BBD_BENCH_NO_FLUSH"): flush.zero_()
@@ -599,7 +651,7 @@ def run_ours(args):
     full = None
     if not args.no_full_step and args.workload == DEFAULT_WORKLOAD:
         try:
-            full = full_step_record(args, dev, world, rank, local, cfg["batch"], H, W, steps=min(args.steps, 10),
+            full = full_step_record(args, dev, world, rank, local, cfg["batch"], H, W, steps=args.steps,
                                     context_legs=False)
         except Exception as exc:  # noqa: BLE001
             full = {"unavailable": f"{type(exc).__name__}: {exc}"}
@@ -671,12 +723,12 @@ def full_step_record(args, dev, world, rank, local, B, H, W, steps, context_legs
     launches = be.launches // 3                               # jittery: the median of three timed loops is reported
     ms, _, loss = sorted(runs)[1]
     nosync_ms = sorted(timed(fused, steps, 1, no_sync=True)[0] for _ in range(3))[1] if world > 1 else None
-    _, e2e_wall, _ = timed(fused, max(10, min(steps, 30)), 2, upload=True)
+    _, e2e_wall, _ = timed(fused, steps, 2, upload=True)
     legs = {}
     for name in (("none", "eager") if context_legs else ("none",)):   # same networks and optimiser, other loss
         torch.manual_seed(1)
         other = FS.StepTrainer(B, H, W, dev, loss=name, ddp=world > 1, local_rank=local)
-        legs[name] = sorted(timed(other, max(5, steps // 2), 3 if i == 0 else 0)[0] for i in range(3))[1]
+        legs[name] = sorted(timed(other, steps, 3 if i == 0 else 0)[0] for i in range(3))[1]
         del other
         torch.cuda.empty_cache()
     n_params = fused.n_params

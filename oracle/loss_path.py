@@ -99,6 +99,52 @@ def disp_to_depth(disp, min_depth, max_depth):
     return scaled, 1 / scaled
 
 
+def rot_from_axisangle(vec):
+    """Axis-angle (n,1,3) -> homogeneous rotation (n,4,4), written element by element into zeros.
+    ``layers.py:61-100``."""
+    angle = torch.norm(vec, 2, 2, True)
+    axis = vec / (angle + 1e-7)
+    ca, sa = torch.cos(angle), torch.sin(angle)
+    C = 1 - ca
+    x, y, z = axis[..., 0].unsqueeze(1), axis[..., 1].unsqueeze(1), axis[..., 2].unsqueeze(1)
+    xs, ys, zs = x * sa, y * sa, z * sa
+    xC, yC, zC = x * C, y * C, z * C
+    xyC, yzC, zxC = x * yC, y * zC, z * xC
+    rot = torch.zeros((vec.shape[0], 4, 4), device=vec.device, dtype=vec.dtype)
+    rot[:, 0, 0] = torch.squeeze(x * xC + ca)
+    rot[:, 0, 1] = torch.squeeze(xyC - zs)
+    rot[:, 0, 2] = torch.squeeze(zxC + ys)
+    rot[:, 1, 0] = torch.squeeze(xyC + zs)
+    rot[:, 1, 1] = torch.squeeze(y * yC + ca)
+    rot[:, 1, 2] = torch.squeeze(yzC - xs)
+    rot[:, 2, 0] = torch.squeeze(zxC - ys)
+    rot[:, 2, 1] = torch.squeeze(yzC + xs)
+    rot[:, 2, 2] = torch.squeeze(z * zC + ca)
+    rot[:, 3, 3] = 1
+    return rot
+
+
+def get_translation_matrix(translation_vector):
+    """Translation (n,1,3) -> homogeneous (n,4,4).  ``layers.py:45-58``."""
+    T = torch.zeros(translation_vector.shape[0], 4, 4, device=translation_vector.device, dtype=translation_vector.dtype)
+    t = translation_vector.contiguous().view(-1, 3, 1)
+    for i in range(4):
+        T[:, i, i] = 1
+    T[:, :3, 3, None] = t
+    return T
+
+
+def transformation_from_parameters(axisangle, translation, invert=False):
+    """(axis-angle, translation) -> 4x4 camera motion.  ``layers.py:25-42``."""
+    R = rot_from_axisangle(axisangle)
+    t = translation.clone()
+    if invert:
+        R = R.transpose(1, 2)
+        t *= -1
+    T = get_translation_matrix(t)
+    return torch.matmul(R, T) if invert else torch.matmul(T, R)
+
+
 # --------------------------------------------------------------------------
 # trainer.py: sub-batch masks
 # --------------------------------------------------------------------------
