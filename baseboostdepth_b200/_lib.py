@@ -55,6 +55,18 @@ class D2DArgs(C.Structure):
                 ("gdisp", fp * MAX_SCALES), ("scratch", fp)]
 
 
+class FrameGradArgs(C.Structure):
+    _fields_ = [("gscale", fp), ("stack_rows", C.c_int32 * MAX_FRAMES), ("coef", fp), ("gpred", fp), ("keys", fp),
+                ("gident", fp), ("gtarget", fp), ("keys_sorted", fp), ("order", fp), ("seg_start", fp),
+                ("gframes", fp * MAX_FRAMES)]
+
+
+class SmoothImgArgs(C.Structure):
+    _fields_ = [("batch", C.c_int32), ("levels", C.c_int32), ("h", C.c_int32 * MAX_SCALES),
+                ("w", C.c_int32 * MAX_SCALES), ("disp", fp * MAX_SCALES), ("img", fp * MAX_SCALES), ("coef", fp),
+                ("gscale", fp), ("gimg", fp * MAX_SCALES)]
+
+
 # every symbol include/bbd_loss.h declares (checked by tests/test_abi.py)
 EXPORTS = [
     "bbd_version", "bbd_last_error_string", "bbd_reproj_tiles", "bbd_ident_forward", "bbd_reproj_fused",
@@ -66,6 +78,7 @@ EXPORTS = [
     "bbd_pose_forward", "bbd_pose_backward", "bbd_grid_sample_forward", "bbd_grid_sample_backward",
     "bbd_grid_sample_dest_keys", "bbd_grid_sample_backward_image",
     "bbd_u8_to_f32", "bbd_loss_combine_forward", "bbd_loss_combine_backward", "bbd_pack_rgba", "bbd_project_coords", "bbd_reproj_kernel_name", "bbd_reproj_finalizes_itself",
+    "bbd_frame_grad", "bbd_frame_grad_stacks", "bbd_smooth_image_grad",
 ]
 
 
@@ -126,7 +139,7 @@ class Backend:
         if self.cuda:
             args = args + (self.stream(),)
         rc = fn(*args)
-        self.launches += {"grid_sample_backward_image": 2}.get(name, 1)
+        self.launches += {"grid_sample_backward_image": 2, "frame_grad": 2, "frame_grad_stacks": 2}.get(name, 1)
         if rc != 0:
             msg = self.dll.bbd_last_error_string().decode() if self.cuda else ""
             raise RuntimeError(f"bbd_{name} failed with code {rc}: {msg}")

@@ -15,7 +15,8 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 SRC = os.path.join(HERE, "csrc", "bbd_kernels.cu")
 OUT = os.path.join(HERE, "libbbd_loss.so")
 DEPS = [os.path.join(HERE, "csrc", f) for f in
-        ("bbd_kernels.cu", "bbd_common.cuh", "bbd_strip.cuh", "bbd_stream.cuh", "bbd_pipe.cuh", "bbd_smooth.cuh", "bbd_ops.cuh")] + [
+        ("bbd_kernels.cu", "bbd_common.cuh", "bbd_strip.cuh", "bbd_stream.cuh", "bbd_pipe.cuh", "bbd_smooth.cuh", "bbd_ops.cuh",
+         "bbd_framegrad.cuh")] + [
     os.path.join(os.path.dirname(HERE), "include", "bbd_loss.h")]
 
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",

@@ -15,6 +15,7 @@
 #include "bbd_strip.cuh"
 #include "bbd_stream.cuh"
 #include "bbd_pipe.cuh"
+#include "bbd_framegrad.cuh"
 
 namespace bbd {
 
@@ -693,6 +694,49 @@ static int grid_for(size_t total, int block) {
   return (int)(g < cap ? (g ? g : 1) : cap);
 }
 
+// ------------------------------------------------------------------------------------------
+// gradients w.r.t. the colour frames (bbd_framegrad.cuh): one thread per pixel, grid-stride
+// ------------------------------------------------------------------------------------------
+__global__ void __launch_bounds__(256) frame_grad_coef_kernel(const bbd_reproj_args a, const bbd_frame_grad_args f) {
+  const int HW = a.height * a.width;
+  const size_t total = (size_t)a.num_scales * a.batch * HW;
+  for (size_t i = blockIdx.x * (size_t)blockDim.x + threadIdx.x; i < total; i += (size_t)gridDim.x * blockDim.x) {
+    const int q = (int)(i % HW), sb = (int)(i / HW);
+    fg_coef_px(a, f, sb / a.batch, sb % a.batch, q / a.width, q % a.width);
+  }
+}
+__global__ void __launch_bounds__(256) frame_grad_pred_kernel(const bbd_reproj_args a, const bbd_frame_grad_args f) {
+  const int HW = a.height * a.width;
+  const size_t total = (size_t)a.batch * HW;
+  for (size_t i = blockIdx.x * (size_t)blockDim.x + threadIdx.x; i < total; i += (size_t)gridDim.x * blockDim.x) {
+    const int p = (int)(i % HW);
+    fg_pred_px(a, f, (int)(i / HW), p / a.width, p % a.width);
+  }
+}
+__global__ void __launch_bounds__(256) frame_grad_stack_kernel(const bbd_reproj_args a, const bbd_frame_grad_args f, int rows) {
+  const int HW = a.height * a.width;
+  const size_t total = (size_t)rows * 3 * HW;
+  for (size_t i = blockIdx.x * (size_t)blockDim.x + threadIdx.x; i < total; i += (size_t)gridDim.x * blockDim.x) {
+    const int p = (int)(i % HW), c = (int)((i / HW) % 3), grow = (int)(i / ((size_t)3 * HW));
+    int slot, row;
+    fg_locate_row(f, grow, slot, row);
+    if (f.gframes[slot]) f.gframes[slot][((size_t)row * 3 + c) * HW + p] = fg_stack_px(a, f, slot, row, c, p);
+  }
+}
+__global__ void __launch_bounds__(256) smooth_image_grad_kernel(const bbd_smooth_img_args a) {
+  const int lvl = blockIdx.z, b = blockIdx.y;
+  if (!a.gimg[lvl]) return;
+  const int h = a.h[lvl], w = a.w[lvl], n = h * w;
+  float* out = a.gimg[lvl] + (size_t)b * 3 * n;
+  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
+    float g[3];
+    smi_px(a, lvl, b, i / w, i % w, g);
+    out[i] = g[0];
+    out[n + i] = g[1];
+    out[2 * n + i] = g[2];
+  }
+}
+
 }  // namespace bbd
 
 using namespace bbd;
@@ -1262,6 +1306,76 @@ int bbd_ssim_backward(int32_t n, int32_t channels, int32_t height, int32_t width
   ssim_grad_kernel<<<grid_for((size_t)n * channels * height * width, 128), 128, 0, (cudaStream_t)stream>>>(
       n * channels, height, width, x, y, gout, gx, gy);
   return check_launch("ssim_grad_kernel");
+}
+
+// what both frame-gradient calls read; sizes and index ranges
+static int frame_grad_check(const bbd_reproj_args* a, const bbd_frame_grad_args* f, const char* who) {
+  static thread_local char msg[128];
+  if (!a || !f || !a->target || !a->depth || !a->inv_K || !a->P || !a->tab.hdr || !a->tab.rep || !a->tab.ident ||
+      !f->gpred || !f->gident) {
+    snprintf(msg, sizeof(msg), "%s: null argument", who);
+    return fail(BBD_E_ARG, msg);
+  }
+  if (a->batch <= 0 || a->height < 2 || a->width < 2 || a->num_scales <= 0) {
+    snprintf(msg, sizeof(msg), "%s: bad size", who);
+    return fail(BBD_E_ARG, msg);
+  }
+  size_t rows = 0;
+  for (int s = 0; s < BBD_MAX_FRAMES; ++s) {
+    if (f->stack_rows[s] < 0) {
+      snprintf(msg, sizeof(msg), "%s: negative stack_rows", who);
+      return fail(BBD_E_RANGE, msg);
+    }
+    rows += (size_t)f->stack_rows[s];
+  }
+  const size_t HW = (size_t)a->height * a->width;
+  if (a->num_scales > BBD_MAX_SCALES || a->max_rep < 1 || a->max_rep > BBD_MAX_REP ||
+      (size_t)a->num_scales * a->batch * a->max_rep * HW >= ((size_t)1 << 31) || rows * HW >= ((size_t)1 << 31) - 1) {
+    snprintf(msg, sizeof(msg), "%s: scales / max_rep / entry count out of range", who);
+    return fail(BBD_E_RANGE, msg);
+  }
+  return 0;
+}
+
+int bbd_frame_grad(const bbd_reproj_args* a, const bbd_frame_grad_args* f, bbd_stream_t stream) {
+  if (int e = frame_grad_check(a, f, "frame_grad")) return e;
+  if (!a->winner || !f->gscale || !f->keys || (!a->no_ssim && !f->coef))
+    return fail(BBD_E_ARG, "frame_grad: winner / gscale / keys / coef missing");
+  cudaStream_t st = (cudaStream_t)stream;
+  const size_t HW = (size_t)a->height * a->width;
+  if (!a->no_ssim)
+    frame_grad_coef_kernel<<<grid_for((size_t)a->num_scales * a->batch * HW, 256), 256, 0, st>>>(*a, *f);
+  frame_grad_pred_kernel<<<grid_for((size_t)a->batch * HW, 256), 256, 0, st>>>(*a, *f);
+  return check_launch("frame_grad kernels");
+}
+
+int bbd_frame_grad_stacks(const bbd_reproj_args* a, const bbd_frame_grad_args* f, bbd_stream_t stream) {
+  if (int e = frame_grad_check(a, f, "frame_grad_stacks")) return e;
+  if (!f->keys_sorted || !f->order || !f->seg_start) return fail(BBD_E_ARG, "frame_grad_stacks: sorted keys / order / seg_start missing");
+  int rows = 0;
+  for (int s = 0; s < BBD_MAX_FRAMES; ++s) rows += f->stack_rows[s];
+  if (rows == 0) return 0;
+  cudaStream_t st = (cudaStream_t)stream;
+  const size_t HW = (size_t)a->height * a->width;
+  const int n_items = (int)((size_t)a->num_scales * a->batch * a->max_rep * HW), n_keys = (int)(rows * HW);
+  gs_segment_kernel<<<grid_for((size_t)n_items + 1, 256), 256, 0, st>>>(f->keys_sorted, n_items, n_keys, f->seg_start);
+  frame_grad_stack_kernel<<<grid_for((size_t)rows * 3 * HW, 256), 256, 0, st>>>(*a, *f, rows);
+  return check_launch("frame_grad_stack_kernel");
+}
+
+int bbd_smooth_image_grad(const bbd_smooth_img_args* a, bbd_stream_t stream) {
+  if (!a || !a->gscale) return fail(BBD_E_ARG, "smooth image gradient: null argument");
+  if (a->levels < 1 || a->levels > BBD_MAX_SCALES || a->batch <= 0 || a->batch > 65535)
+    return fail(BBD_E_RANGE, "smooth image gradient: bad level count / batch");
+  int mx = 1;
+  for (int l = 0; l < a->levels; ++l) {
+    if (!a->gimg[l]) continue;
+    if (!a->disp[l] || !a->img[l] || a->h[l] < 2 || a->w[l] < 2) return fail(BBD_E_ARG, "smooth image gradient: bad level");
+    mx = std::max(mx, a->h[l] * a->w[l]);
+  }
+  dim3 grid(std::min((mx + 255) / 256, 64), a->batch, a->levels);
+  smooth_image_grad_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(*a);
+  return check_launch("smooth_image_grad_kernel");
 }
 
 }  // extern "C"

@@ -6,7 +6,8 @@ over ``generate_images_pred`` (``trainer.py:444-475``) and ``compute_losses``
 per-pixel minimum, smoothness -- forward *and* backward -- in a dozen kernel
 launches (the small ones on helper streams next to the identity pre-pass), and returns the per-scale reprojection means and smoothness terms as
 differentiable tensors.  Gradients flow to the disparities and to the packed
-projection matrices ``P = (K @ T)[:, :3, :]``.
+projection matrices ``P = (K @ T)[:, :3, :]``, and to the colour frames (target,
+source stacks, pyramid levels) that require one (``_frame_backward``).
 
 Because every loss term is a mean with a weight known in advance, the kernels
 produce the unit gradients during the forward launch; ``backward`` only folds
@@ -151,13 +152,15 @@ def disps_key(disps):
     return tuple((d.data_ptr(), tuple(d.shape), d._version) for d in disps)
 
 
-def start_side_branch(be, disps, pyramid, bhw, min_depth, max_depth, sql, need_grad, timers=None):
+def start_side_branch(be, disps, pyramid, bhw, min_depth, max_depth, sql, need_grad, timers=None, need_coef=False):
     """Launch disparity -> depth (reference ``trainer.py:456`` + ``layers.py:13-22``) and the smoothness
     kernels (``trainer.py:560-564``) for one step.  They depend only on the disparities and the colour
     pyramid, are small and latency-bound, and therefore run on a helper stream between a fork and a
     join event (graph-capturable) while the launch stream goes on with the pose packing, the noise
     draw and the identity pre-pass; ``_FusedLoss.forward`` waits for ``join`` before the fused kernel.
-    Every buffer is allocated here on the launch stream, before the fork."""
+    Every buffer is allocated here on the launch stream, before the fork.  ``need_coef``: keep the
+    per-(level, sample) normalisation scalars even without disparity gradients (the pyramid's gradient
+    reads them)."""
     B, H, W = bhw
     S = len(disps)
     assert 1 <= S <= _lib.MAX_SCALES
@@ -205,7 +208,7 @@ def start_side_branch(be, disps, pyramid, bhw, min_depth, max_depth, sql, need_g
     sa.scratch, sa.loss = scratch.data_ptr(), smooth.data_ptr()
     keep.append(scratch)
     # the mean-normalisation of the smoothness gradient is finished by the disparity backward (one pass less)
-    coef = torch.empty(S, B, 2, **f32) if need_grad else None
+    coef = torch.empty(S, B, 2, **f32) if need_grad or need_coef else None
     if coef is not None:
         sa.defer_norm, sa.coef = 1, coef.data_ptr()
 
@@ -232,18 +235,21 @@ def start_side_branch(be, disps, pyramid, bhw, min_depth, max_depth, sql, need_g
 
 
 class _FusedLoss(torch.autograd.Function):
-    """(P, disp_0..disp_{S-1}) -> (reproj[S], smooth[S]); everything else is closed over."""
+    """(P, disp_0..disp_{S-1}, target, frame stacks in plan.frames order, pyramid_0..pyramid_{S-1})
+    -> (reproj[S], smooth[S]); inv_K and the noise are closed over."""
 
     @staticmethod
-    def forward(ctx, cfg, P, *disps):
+    def forward(ctx, cfg, P, *tensors):
         be: _lib.Backend = cfg["backend"]
         plan: LossPlan = cfg["plan"]
         target, frames, inv_K = cfg["target"], cfg["frames"], cfg["inv_K"]
         noise, pyramid = cfg["noise"], cfg["pyramid"]
+        disps = tensors[:len(pyramid)]
         B, _, H, W = target.shape
         S = len(disps)
         dev = target.device
         need_grad = bool(cfg["need_grad"])
+        frame_grad = bool(cfg["frame_grad"])
         f32 = dict(device=dev, dtype=torch.float32)
         be.check_device(target, inv_K, P, *disps, *pyramid, *noise.values(), *frames.values())
         assert plan.batch == B and P.shape == (plan.n_pose, 3, 4), (P.shape, plan.n_pose)
@@ -254,6 +260,7 @@ class _FusedLoss(torch.autograd.Function):
         inv_K = inv_K.contiguous()
         tab = _tables(plan, dev)
         frame_arr, keep = _frame_ptrs(plan, frames, H, W)
+        frames_c = list(keep)
         rgba_arr, rgba_keep = rgba_buffers(keep, H, W) if stream_eligible(plan) else (None, [])
 
         # 1 + 5. disparity -> depth and smoothness: on the helper stream (started here unless the caller
@@ -261,15 +268,17 @@ class _FusedLoss(torch.autograd.Function):
         # (popped: `smooth` becomes an output of this node, and an output reachable from ctx would be a
         # reference cycle that keeps the autograd graph -- and its AccumulateGrad nodes -- alive)
         pre = cfg.pop("pre", None)
-        if pre is None or pre["disps"] != disps_key(disps) or (need_grad and not pre["gsm"]):
+        pyr_grad = frame_grad and any(p.requires_grad for p in pyramid)
+        if (pre is None or pre["disps"] != disps_key(disps) or (need_grad and not pre["gsm"])
+                or (pyr_grad and pre["coef"] is None)):
             pre = start_side_branch(be, disps, pyramid, (B, H, W), cfg["min_depth"], cfg["max_depth"], cfg["sql"],
-                                    need_grad, timers=cfg.get("timers"))
+                                    need_grad, timers=cfg.get("timers"), need_coef=pyr_grad)
         disps_c, d2d, depth, gsm, smooth, join = (pre[k] for k in ("disps_c", "d2d", "depth", "gsm", "smooth", "join"))
         keep.extend(pre["keep"])
 
         # 2. identity pre-pass (once per step)
         ident_min = torch.empty(B, H, W, **f32)
-        want_winner = bool(cfg["want_winner"])
+        want_winner = bool(cfg["want_winner"]) or frame_grad   # the frame gradient differentiates these winners
         ident_arg = torch.empty(B, H, W, device=dev, dtype=torch.uint8) if want_winner else None
         ia = _lib.IdentArgs()
         ia.batch, ia.height, ia.width, ia.no_ssim = B, H, W, int(cfg["no_ssim"])
@@ -337,6 +346,10 @@ class _FusedLoss(torch.autograd.Function):
         del rgba_keep   # consumed by the fused kernel (stream-ordered: the allocator may reuse it from here on)
         ctx.keep = (disps_c, depth, gdepth, gpose, gsm, pre["coef"])
         ctx.aux = {"depth": depth, "ident_min": ident_min, "ident_arg": ident_arg, "winner": winner}
+        ctx.frame_grad = frame_grad
+        if frame_grad:
+            # what the frame gradient reads again: the argument block of the fused kernel and the buffers it points at
+            ctx.frame_keep = (ra, target, inv_K, Pc, frames_c, pre["keep"][:S], winner, ident_arg, ident_min)
         cfg["aux"] = ctx.aux
         return reproj, smooth
 
@@ -345,10 +358,15 @@ class _FusedLoss(torch.autograd.Function):
         cfg = ctx.cfg
         be: _lib.Backend = cfg["backend"]
         disps_c, depth, gdepth, gpose, gsm, coef = ctx.keep
-        if gdepth is None:
-            raise RuntimeError("bbd: fused loss was evaluated with need_grad=False")
         g_reproj = g_reproj.contiguous().float()
         g_smooth = g_smooth.contiguous().float()
+        S = len(disps_c)
+        frame_grads = _frame_backward(ctx, be, g_reproj, g_smooth, S) if ctx.frame_grad else (None,) * (
+            len(ctx.needs_input_grad) - 2 - S)
+        if gdepth is None:
+            if not ctx.frame_grad:
+                raise RuntimeError("bbd: fused loss was evaluated with need_grad=False")
+            return (None, None) + (None,) * S + frame_grads
         gP = torch.einsum("s,spij->pij", g_reproj, gpose) if ctx.needs_input_grad[1] else None
         d2d = ctx.d2d
         gdisps = [torch.empty_like(d) for d in disps_c]
@@ -362,7 +380,6 @@ class _FusedLoss(torch.autograd.Function):
         scratch = torch.empty(max(1, be.value("d2d_scratch_floats", C.byref(d2d))), device=gdepth.device,
                               dtype=torch.float32)
         d2d.scratch = scratch.data_ptr()
-        S = len(gdisps)
         full_res_first = S > 1 and tuple(disps_c[0].shape[-2:]) == tuple(depth.shape[-2:])
         timers = cfg.get("timers")
         if timers is not None and be.cuda:
@@ -387,7 +404,59 @@ class _FusedLoss(torch.autograd.Function):
         if timers is not None and be.cuda:
             tb1.record()
             timers["disp_to_depth_backward"] = (tb0, tb1)
-        return (None, gP) + tuple(gdisps)
+        return (None, gP) + tuple(gdisps) + frame_grads
+
+
+def _frame_backward(ctx, be, g_reproj, g_smooth, S):
+    """Gradients of (target, frame stacks..., pyramid levels...) as ``ctx.needs_input_grad`` asks for them:
+    bbd_frame_grad, a stable sort of its keys, bbd_frame_grad_stacks, and bbd_smooth_image_grad."""
+    cfg = ctx.cfg
+    plan: LossPlan = cfg["plan"]
+    ra, target, inv_K, Pc, frames_c, pyr_c, winner, ident_arg, ident_min = ctx.frame_keep
+    needs = ctx.needs_input_grad[2 + S:]
+    n_f = len(frames_c)
+    need_target, need_frames, need_pyr = needs[0], needs[1:1 + n_f], needs[1 + n_f:]
+    B, _, H, W = target.shape
+    dev, HW = target.device, H * W
+    f32 = dict(device=dev, dtype=torch.float32)
+    gtarget, gframes, gpyr = None, [None] * n_f, [None] * S
+    if need_target or any(need_frames):
+        fa = _lib.FrameGradArgs()
+        fa.gscale = g_reproj.data_ptr()
+        for slot, t in enumerate(frames_c):
+            fa.stack_rows[slot] = t.shape[0]
+        coef = None if cfg["no_ssim"] else torch.empty(S, B, 3, 6, H, W, **f32)
+        gpred = torch.empty(S, B, plan.max_rep, 3, H, W, **f32)
+        keys = torch.empty(S * B * plan.max_rep * HW, device=dev, dtype=torch.int32)
+        gident = torch.empty(B, _lib.MAX_IDENT, 3, H, W, **f32)
+        gtarget = torch.empty(B, 3, H, W, **f32) if need_target else None
+        fa.coef, fa.gpred, fa.keys = _lib.ptr(coef), gpred.data_ptr(), keys.data_ptr()
+        fa.gident, fa.gtarget = gident.data_ptr(), _lib.ptr(gtarget)
+        be.call("frame_grad", C.byref(ra), C.byref(fa))
+        if any(need_frames):
+            keys_sorted, order = torch.sort(keys, stable=True)
+            order = order.to(torch.int32)
+            seg = torch.empty(sum(t.shape[0] for t in frames_c) * HW + 1, device=dev, dtype=torch.int32)
+            fa.keys_sorted, fa.order, fa.seg_start = keys_sorted.data_ptr(), order.data_ptr(), seg.data_ptr()
+            for slot, t in enumerate(frames_c):
+                if need_frames[slot]:
+                    gframes[slot] = torch.empty_like(t) if t.numel() else torch.zeros_like(t)
+                    fa.gframes[slot] = _lib.ptr(gframes[slot]) if t.numel() else None
+            be.call("frame_grad_stacks", C.byref(ra), C.byref(fa))
+    if any(need_pyr):
+        _, _, _, _, _, coef_s = ctx.keep
+        disps_c = ctx.keep[0]
+        sa = _lib.SmoothImgArgs()
+        sa.batch, sa.levels = B, S
+        sa.coef, sa.gscale = coef_s.data_ptr(), g_smooth.data_ptr()
+        for l in range(S):
+            sa.h[l], sa.w[l] = disps_c[l].shape[2], disps_c[l].shape[3]
+            sa.disp[l], sa.img[l] = disps_c[l].data_ptr(), pyr_c[l].data_ptr()
+            if need_pyr[l]:
+                gpyr[l] = torch.empty_like(pyr_c[l])
+                sa.gimg[l] = gpyr[l].data_ptr()
+        be.call("smooth_image_grad", C.byref(sa))
+    return (gtarget,) + tuple(gframes) + tuple(gpyr)
 
 
 def fused_losses(plan: LossPlan, target: torch.Tensor, frames: Dict, disps: Sequence[torch.Tensor],
@@ -406,10 +475,14 @@ def fused_losses(plan: LossPlan, target: torch.Tensor, frames: Dict, disps: Sequ
     be = backend if backend is not None else _lib.cuda_backend()
     if need_grad is None:
         need_grad = torch.is_grad_enabled() and (P.requires_grad or any(d.requires_grad for d in disps))
+    frame_list = [frames[f] for f in plan.frames]
+    pyramid = list(pyramid)
+    frame_grad = torch.is_grad_enabled() and any(t.requires_grad for t in [target] + frame_list + pyramid)
     cfg = dict(backend=be, plan=plan, target=target, frames=frames, inv_K=inv_K, noise=noise,
-               pyramid=list(pyramid), min_depth=min_depth, max_depth=max_depth, no_ssim=no_ssim, sql=sql,
-               noise_scale=noise_scale, want_winner=want_winner, need_grad=need_grad, timers=timers, pre=pre)
-    reproj, smooth = _FusedLoss.apply(cfg, P, *disps)
+               pyramid=pyramid, min_depth=min_depth, max_depth=max_depth, no_ssim=no_ssim, sql=sql,
+               noise_scale=noise_scale, want_winner=want_winner, need_grad=need_grad, frame_grad=frame_grad,
+               timers=timers, pre=pre)
+    reproj, smooth = _FusedLoss.apply(cfg, P, *disps, target, *frame_list, *pyramid)
     return reproj, smooth, cfg["aux"]
 
 

@@ -214,25 +214,35 @@ class _Smooth(torch.autograd.Function):
         loss = torch.empty(1, device=d.device, dtype=torch.float32)
         sa.scratch, sa.loss = scratch.data_ptr(), loss.data_ptr()
         be.call("smooth_fused", C.byref(sa))
-        ctx.save_for_backward(gdisp)
+        ctx.save_for_backward(gdisp, d, im)
         return loss[0]
 
     @staticmethod
     def backward(ctx, g):
-        (gdisp,) = ctx.saved_tensors
-        return gdisp * g, None
+        gdisp, d, im = ctx.saved_tensors
+        gimg = None
+        if ctx.needs_input_grad[1]:
+            be = _backend()
+            B, _, h, w = d.shape
+            gs = g.detach().reshape(1).contiguous().float()
+            gimg = torch.empty_like(im)
+            ia = _lib.SmoothImgArgs()
+            ia.batch, ia.levels = B, 1
+            ia.h[0], ia.w[0] = h, w
+            ia.disp[0], ia.img[0], ia.gimg[0] = d.data_ptr(), im.data_ptr(), gimg.data_ptr()
+            ia.coef, ia.gscale = None, gs.data_ptr()     # no normalisation: r = 1
+            be.call("smooth_image_grad", C.byref(ia))
+        return gdisp * g, gimg
 
 
 def get_smooth_loss(disp, img):
     """Edge-aware smoothness of a disparity image, 0-d tensor.  Reference ``layers.py:203-216``.
 
-    One fused forward+backward pass (the gradient w.r.t. ``disp`` is produced with the value;
-    ``img`` carries no gradient in the trainer and none is provided).  The trainer passes the
-    mean-normalised disparity (``trainer.py:560-563``); the fused path folds that
+    One fused forward+backward pass (the gradient w.r.t. ``disp`` is produced with the value).
+    When ``img`` requires grad, the backward adds one gather kernel for its gradient.  The trainer
+    passes the mean-normalised disparity (``trainer.py:560-563``); the fused path folds that
     normalisation into the same kernel (``normalize=1``).
     """
-    if img.requires_grad:
-        raise NotImplementedError("bbd get_smooth_loss: gradient w.r.t. the image is not provided")
     return _Smooth.apply(disp, img)
 
 

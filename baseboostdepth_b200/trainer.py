@@ -139,8 +139,10 @@ def loss_step(inputs, outputs, opt, plan: Optional[LossPlan] = None, noise=None,
         noise_scale = 0.00001
     else:
         noise_scale = 1.0
+    # (a colour level that requires grad also needs the smoothness normalisation scalars)
     pre = start_side_branch(be, disps, pyramid, (B, H, W), opt.min_depth, opt.max_depth, getattr(opt, "SQL", False),
-                            torch.is_grad_enabled(), timers=timers)
+                            torch.is_grad_enabled(), timers=timers,
+                            need_coef=torch.is_grad_enabled() and any(p.requires_grad for p in pyramid))
 
     T = _frame_poses(plan, inputs, outputs, "cam_T_cam", row_masks)
     T_err = _frame_poses(plan, inputs, outputs, "cam_T_cam_error", row_masks) if plan.decomp else None

@@ -146,6 +146,35 @@ const char* bbd_reproj_kernel_name(const bbd_reproj_args* a);
 /* loss (S) = sum(loss_part)/(B*H*W); gpose (S,num_pose,3,4) = sum over tiles. */
 int bbd_reproj_finalize(const bbd_reproj_args* a, float* loss, float* gpose, bbd_stream_t stream);
 
+/* ---- gradient of the fused loss w.r.t. the colour frames -------------------
+ * trainer.py:477-486 + :525-557 under autograd with the target ("color",0,0) and the source stacks
+ * ("color",f,0) requiring grad: only the per-pixel winner's photometric term is differentiated, the winners
+ * being the ones the forward wrote to bbd_reproj_args.winner (which, with ident_arg, this needs; depth, inv_K,
+ * P, target, frames and tab as in the forward).  Two calls around a caller-side STABLE sort:
+ *   bbd_frame_grad         writes gtarget, gident, gpred and keys (coef is scratch);
+ *   (caller)               sorts keys -> keys_sorted with order = the permutation as int32 (n_items entries);
+ *   bbd_frame_grad_stacks  gathers, per stack pixel, the transposed bilinear warps of every scale, candidate
+ *                          and decomp twin that sampled it (four runs of the sorted order, as
+ *                          bbd_grid_sample_backward_image) plus the identity-source gradients; seg_start is
+ *                          scratch.  Every gframes[f] given is fully written (zero where nothing reads it).
+ * Sums run in a fixed order and use no atomics: the result is bit-reproducible.
+ * n_items = num_scales*B*max_rep*H*W; n_keys = (sum of stack_rows)*H*W; both must stay below 2^31. */
+typedef struct bbd_frame_grad_args {
+  const float* gscale;                  /* (S) device: upstream gradient of the per-scale reprojection means */
+  int32_t stack_rows[BBD_MAX_FRAMES];   /* rows of each frame stack (0 for an empty or absent slot) */
+  float* coef;                          /* (S,B,3,6,H,W) scratch; may be NULL under no_ssim */
+  float* gpred;                         /* (S,B,max_rep,3,H,W): d loss / d warped candidate (read where keyed) */
+  int32_t* keys;                        /* (n_items): stack row * H*W + north-west tap, or n_keys (no gradient) */
+  float* gident;                        /* (B,BBD_MAX_IDENT,3,H,W): identity-source gradients, rows < n_ident */
+  float* gtarget;                       /* (B,3,H,W) or NULL */
+  const int32_t* keys_sorted;           /* bbd_frame_grad_stacks only: (n_items) */
+  const int32_t* order;                 /* bbd_frame_grad_stacks only: (n_items) */
+  int32_t* seg_start;                   /* bbd_frame_grad_stacks only: n_keys + 1 int32 of scratch */
+  float* gframes[BBD_MAX_FRAMES];       /* bbd_frame_grad_stacks only: (stack_rows[f],3,H,W) or NULL to skip */
+} bbd_frame_grad_args;
+int bbd_frame_grad(const bbd_reproj_args* a, const bbd_frame_grad_args* f, bbd_stream_t stream);
+int bbd_frame_grad_stacks(const bbd_reproj_args* a, const bbd_frame_grad_args* f, bbd_stream_t stream);
+
 /* ---- camera motion from network outputs ---------------------------------------
  * layers.py:25-100: transformation_from_parameters(axisangle, translation, invert) =
  * get_translation_matrix(t) @ rot_from_axisangle(v), or R^T @ T(-t) when invert.  One thread per
@@ -198,6 +227,19 @@ typedef struct bbd_smooth_args {
 } bbd_smooth_args;
 size_t bbd_smooth_scratch_floats(int32_t batch, int32_t levels, const int32_t* h, const int32_t* w);
 int bbd_smooth_fused(const bbd_smooth_args* a, bbd_stream_t stream);
+/* Gradient of the smoothness terms w.r.t. the colour levels (layers.py:203-216 under autograd): per pixel, a
+ * gather over its four edges.  gimg[l] = gscale[l] * d loss[l] / d img_l, with the normalisation scalar
+ * 1/(mean+1e-7) read from coef[l,b,0] as bbd_smooth_fused leaves it (defer_norm), or 1 when coef is NULL. */
+typedef struct bbd_smooth_img_args {
+  int32_t batch, levels;
+  int32_t h[BBD_MAX_SCALES], w[BBD_MAX_SCALES];
+  const float* disp[BBD_MAX_SCALES]; /* (B,1,h,w) */
+  const float* img[BBD_MAX_SCALES];  /* (B,3,h,w) */
+  const float* coef;                 /* (levels,B,2) or NULL */
+  const float* gscale;               /* (levels) device: upstream gradient of each level's loss */
+  float* gimg[BBD_MAX_SCALES];       /* (B,3,h,w), or NULL to skip the level */
+} bbd_smooth_img_args;
+int bbd_smooth_image_grad(const bbd_smooth_img_args* a, bbd_stream_t stream);
 
 /* ---- disparity -> full-resolution depth, and back ---------------------------
  * trainer.py:456-461 for every scale of a step: F.interpolate(bilinear,
