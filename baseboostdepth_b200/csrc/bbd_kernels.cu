@@ -10,34 +10,19 @@
 #include <algorithm>
 #include <string.h>
 
-#include "bbd_ops.cuh"
-#include "bbd_smooth.cuh"
-#include "bbd_strip.cuh"
-#include "bbd_stream.cuh"
+#include "bbd_launch.cuh"
 #include "bbd_pipe.cuh"
 #include "bbd_framegrad.cuh"
 
 namespace bbd {
 
-// Identity pre-pass and fused loss share one tile geometry: 28x16 target pixels per block of 6
-// warps, lanes = columns (bbd_strip.cuh).  With two warped candidates a block needs 64 KB of shared
-// memory -> 3 blocks (18 warps) per SM at 96 registers per thread.  Fewer, fatter warps beat 8 warps
-// at 80 registers: the kernel gains from instruction-level parallelism inside a warp (four rows of
-// gathers in flight in the warp phase, two rows walked together in the backward), not from more
-// resident warps (profiles/README.md lists the measured variants).
-#ifndef BBD_TILE_H
-#define BBD_TILE_H 16
-#endif
+// resident blocks per SM of the tile kernels (tile geometry SCfg: bbd_launch.cuh)
 #ifndef BBD_MIN_BLOCKS
 #define BBD_MIN_BLOCKS 3
-#endif
-#ifndef BBD_WARPS
-#define BBD_WARPS 6
 #endif
 #ifndef BBD_SCATTER_REDUCE
 #define BBD_SCATTER_REDUCE 1
 #endif
-using SCfg = StripCfg<BBD_TILE_H, BBD_WARPS>;
 
 static thread_local char g_err[256] = "";
 
@@ -206,9 +191,6 @@ __global__ void __launch_bounds__(SCfg::NT, BBD_MIN_BLOCKS) reproj_kernel(const 
 #ifndef BBD_STREAM_WARPS
 #define BBD_STREAM_WARPS 1  // one warp per block: every branch on the unit index is provably warp-uniform,
                             // so the shuffles need no WARPSYNC / ENDCOLLECTIVE brackets
-#endif
-#ifndef BBD_STREAM_MINB
-#define BBD_STREAM_MINB 8
 #endif
 template <int K, bool GRAD, bool MULTI, bool WING = false>
 __global__ void __launch_bounds__(BBD_STREAM_WARPS * 32, BBD_STREAM_MINB) reproj_stream_kernel(const bbd_reproj_args a, int n_units, int part_stride, int seg_rows) {
@@ -741,55 +723,6 @@ __global__ void __launch_bounds__(256) smooth_image_grad_kernel(const bbd_smooth
 
 using namespace bbd;
 
-static int tile_parts(int height, int width) {
-  return ((width + SCfg::TW - 1) / SCfg::TW) * ((height + SCfg::TH - 1) / SCfg::TH);
-}
-// slots per (scale, sample) in loss_part / gpose_part: enough for either kernel
-extern "C" int bbd_reproj_tiles(int32_t height, int32_t width) {
-  return std::max(tile_parts(height, width), std::max(StreamGeo::strips(width) * stream_max_segs(height), StreamGeoM::units(height, width)));
-}
-
-// Which kernel serves these arguments (the finalize step must agree with the fused launch).
-static bool use_stream(const bbd_reproj_args* a) {
-  if (a->force_tile || a->min_rep < 1 || a->max_rep > BBD_MAX_REP) return false;
-  if (BBD_STREAM_ASYNC && a->max_rep > 2) return false;
-  bool any = false;
-  for (int f = 0; f < BBD_MAX_FRAMES; ++f) {
-    if (a->frames[f] && !a->frames_rgba[f]) return false;
-    any = any || a->frames_rgba[f];
-  }
-  return any;
-}
-// resident warps of the one-warp streaming form on this device (8 per SM: 224-243 registers per thread)
-static int stream_slots() {
-  static int slots = 0;
-  if (!slots) {
-    int dev = 0, sms = 148;
-    if (cudaGetDevice(&dev) == cudaSuccess) cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-    slots = sms * BBD_STREAM_MINB;
-  }
-  return slots;
-}
-static int seg_rows_for(const bbd_reproj_args* a) {
-  if (a->max_rep > 2) return stream_seg_rows_uneven(a->height, a->width, a->num_scales * a->batch, stream_slots());
-  return stream_seg_rows(a->height, a->width, a->num_scales * a->batch, stream_slots());
-}
-// The many-candidate form with gradients runs as two launches when the caller provides the winner plane: a forward-only
-// selection launch (twelve warps per SM) and a gradient launch that reads the winners (tall segments).
-static bool split_multi(const bbd_reproj_args* a) {
-  return use_stream(a) && a->max_rep > 2 && a->need_grad && a->winner != nullptr;
-}
-// slots of loss_part / gpose_part a launch fills per (scale, sample): the two can differ in the split form
-static int parts_used(const bbd_reproj_args* a, bool grad_parts) {
-  if (!use_stream(a)) return tile_parts(a->height, a->width);
-  if (a->max_rep > 2 && !(grad_parts && split_multi(a))) return StreamGeoM::units(a->height, a->width);
-  const int rh = seg_rows_for(a);
-  return StreamGeo::strips(a->width) * ((a->height + rh - 1) / rh);
-}
-
-#ifndef BBD_STREAM_TMA
-#define BBD_STREAM_TMA (!BBD_STREAM_ASYNC)
-#endif
 // cuTensorMapEncodeTiled through the runtime's driver entry point (no link against libcuda)
 typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
                                   const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
@@ -819,30 +752,28 @@ static bool make_row_map(CUtensorMap* m, const float* base, int W, int H, long p
              CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
 }
 
-// The pipelined (three-warp) form is an opt-in variant for the single-sweep case (BBD_PIPE=1 in the environment or
-// -DBBD_USE_PIPE=1): parity-green on the B200, but measured slower than the one-warp streaming form (0.453 against
-// 0.418 ms: its three stages are unequal, the gather warp is busy 84 % of the time, the backward warp 53 % --
-// profiles/README.md), so the streaming form stays the default.
-#ifndef BBD_USE_PIPE
-#define BBD_USE_PIPE 0
-#endif
-static bool use_pipe() {
-  const char* e = getenv("BBD_PIPE");  // read per launch: tests switch forms inside one process
-  return e ? (e[0] != '0') : (BBD_USE_PIPE != 0);
+static int device_sms() {
+  static int sms = 0;
+  if (!sms) {
+    int dev = 0;
+    sms = 148;
+    if (cudaGetDevice(&dev) == cudaSuccess) cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+  }
+  return sms;
 }
+// The facts of the current device the launch decisions of the fused loss (bbd_launch.cuh) depend on.
+static LaunchDevice device_facts() { return {device_sms(), encode_tiled() != nullptr, pipe_requested()}; }
 
-template <int K, bool GRAD, bool MULTI, bool WING = false>
-static int launch_stream(const bbd_reproj_args* a, cudaStream_t stream) {
-  const int n_units = a->num_scales * a->batch * parts_used(a, WING);
+template <int K, bool GRAD, bool MULTI, bool WING>
+static int launch_stream(const bbd_reproj_args* a, const ReprojLaunch& L, const KernelLaunch& l, cudaStream_t stream) {
+  const int n_units = l.units, seg_rows = l.seg_rows, stride = L.stride;
   const int blocks = (n_units + BBD_STREAM_WARPS - 1) / BBD_STREAM_WARPS;
-  const int seg_rows = (MULTI && !WING) ? BBD_STREAM_RHM : seg_rows_for(a);
-  const int stride = bbd_reproj_tiles(a->height, a->width);
 #if BBD_STREAM_TMA
   CUtensorMap tt, td, ti;
-  if (make_row_map(&tt, a->target, a->width, a->height, 3L * a->batch, 3) &&
+  if (L.tma && make_row_map(&tt, a->target, a->width, a->height, 3L * a->batch, 3) &&
       make_row_map(&td, a->depth, a->width, a->height, (long)a->num_scales * a->batch, 1) &&
       make_row_map(&ti, a->ident_min, a->width, a->height, a->batch, 1)) {
-    if (!MULTI && use_pipe()) {
+    if (L.form == REPROJ_PIPE) {
       static bool configured_p = false;
       constexpr size_t smem_p = (size_t)PipeSmem<K, GRAD>::FLOATS * sizeof(float);
       if (!configured_p) {
@@ -864,7 +795,7 @@ static int launch_stream(const bbd_reproj_args* a, cudaStream_t stream) {
     return check_launch("reproj_stream_tma_kernel");
   }
 #endif
-  // widths that are not a multiple of four floats (or unaligned planes) cannot be described to the TMA unit
+  // planes the TMA unit cannot describe, or no tensor-map encoder: plain loads
   static bool configured = false;
   constexpr size_t smem = (size_t)BBD_STREAM_WARPS * StreamSmem<K, false, MULTI, GRAD, MULTI && !WING>::FLOATS * sizeof(float);
   if (!configured) {
@@ -884,14 +815,11 @@ const char* bbd_last_error_string(void) { return g_err; }
 int bbd_ident_forward(const bbd_ident_args* a, bbd_stream_t stream) {
   if (!a || !a->target || !a->ident_min || !a->tab.hdr || !a->tab.ident) return fail(BBD_E_ARG, "ident: null argument");
   if (a->batch <= 0 || a->height < 2 || a->width < 2) return fail(BBD_E_ARG, "ident: bad size");
-  if (!a->force_tile) {
+  const IdentLaunch L = ident_launch(*a, device_sms());
+  if (L.stream) {
     RgbaPtrs rp;
     for (int f = 0; f < BBD_MAX_FRAMES; ++f) rp.p[f] = a->frames_rgba[f];
-    int dev = 0, sms = 148;
-    if (cudaGetDevice(&dev) == cudaSuccess) cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-    const int seg_rows = ident_seg_rows(a->height, a->width, a->batch, sms * 16);
-    const int n_units = a->batch * IdentGeo::strips(a->width) * ((a->height + seg_rows - 1) / seg_rows);
-    ident_stream_kernel<<<n_units, 32, 0, (cudaStream_t)stream>>>(*a, rp, n_units, seg_rows);
+    ident_stream_kernel<<<L.units, 32, 0, (cudaStream_t)stream>>>(*a, rp, L.units, L.seg_rows);
     return check_launch("ident_stream_kernel");
   }
   dim3 grid((a->width + SCfg::TW - 1) / SCfg::TW, (a->height + SCfg::TH - 1) / SCfg::TH, a->batch);
@@ -912,22 +840,19 @@ int bbd_reproj_fused(const bbd_reproj_args* a, bbd_stream_t stream) {
   if (a->need_grad && (!a->gpose_part || !a->gdepth)) return fail(BBD_E_ARG, "reproj: gradient buffers missing");
   if (a->batch <= 0 || a->height < 2 || a->width < 2 || a->num_scales <= 0) return fail(BBD_E_ARG, "reproj: bad size");
   if (a->max_rep < 1 || a->max_rep > BBD_MAX_REP) return fail(BBD_E_RANGE, "reproj: max_rep out of range");
-  if (a->tickets && !bbd_reproj_finalizes_itself(a)) return fail(BBD_E_ARG, "reproj: tickets given but pair_sum / loss_out / gpose_out missing or tile kernel selected");
-  if (use_stream(a)) {
-    cudaStream_t st = (cudaStream_t)stream;
-    if (a->max_rep == 1) return a->need_grad ? launch_stream<1, true, false>(a, st) : launch_stream<1, false, false>(a, st);
-    if (a->max_rep == 2) return a->need_grad ? launch_stream<2, true, false>(a, st) : launch_stream<2, false, false>(a, st);
-#if !BBD_STREAM_ASYNC
-    if (split_multi(a)) {  // selection round, then the gradient round reading a->winner
-      if (int rc = launch_stream<2, false, true>(a, st)) return rc;
-      return launch_stream<2, true, true, true>(a, st);
+  const ReprojLaunch L = reproj_launch(*a, device_facts());
+  if (a->tickets && !L.finalizes_itself) return fail(BBD_E_ARG, "reproj: tickets given but pair_sum / loss_out / gpose_out missing or tile kernel selected");
+  if (L.form != REPROJ_TILE) {
+    for (int i = 0; i < L.n_launches; ++i) {  // the many-candidate form with the winner plane: selection, then gradient round
+      const KernelLaunch& l = L.launch[i];
+      const int rc = with_stream_instance(L, l, [&](auto k, auto grad, auto multi, auto wing) {
+        return launch_stream<decltype(k)::value, decltype(grad)::value, decltype(multi)::value, decltype(wing)::value>(a, L, l, (cudaStream_t)stream);
+      });
+      if (rc) return rc;
     }
-    return a->need_grad ? launch_stream<2, true, true>(a, st) : launch_stream<2, false, true>(a, st);
-#endif
+    return 0;
   }
-  // keep every candidate's warped tile resident while that still allows three blocks per SM
-  const bool keep = StripSmem<SCfg>::floats(a->max_rep) * sizeof(float) <= 75 * 1024;
-  const size_t smem = StripSmem<SCfg>::floats(keep ? a->max_rep : 1) * sizeof(float);
+  const size_t smem = L.tile_smem;
   if (smem > 227 * 1024) return fail(BBD_E_RANGE, "reproj: shared memory budget exceeded");
   dim3 grid((a->width + SCfg::TW - 1) / SCfg::TW, (a->height + SCfg::TH - 1) / SCfg::TH, a->num_scales * a->batch);
   static size_t configured[4] = {0, 0, 0, 0};  // largest dynamic shared-memory size granted per variant
@@ -940,56 +865,37 @@ int bbd_reproj_fused(const bbd_reproj_args* a, bbd_stream_t stream) {
     }
     kern<<<grid, SCfg::NT, smem, (cudaStream_t)stream>>>(*a);
   };
-  if (a->need_grad) {
-    if (keep) launch(reproj_kernel<true, true>, 0); else launch(reproj_kernel<true, false>, 1);
+  if (L.launch[0].grad) {
+    if (L.keep) launch(reproj_kernel<true, true>, 0); else launch(reproj_kernel<true, false>, 1);
   } else {
-    if (keep) launch(reproj_kernel<false, true>, 2); else launch(reproj_kernel<false, false>, 3);
+    if (L.keep) launch(reproj_kernel<false, true>, 2); else launch(reproj_kernel<false, false>, 3);
   }
   if (rc) return rc;
   return check_launch("reproj_kernel");
 }
 
-int bbd_reproj_finalizes_itself(const bbd_reproj_args* a) {
-  return a && use_stream(a) && a->max_rep <= 2 && a->tickets && a->pair_sum && a->loss_out && (!a->need_grad || a->gpose_out) ? 1 : 0;
-}
+int bbd_reproj_tiles(int32_t height, int32_t width) { return reproj_slots(height, width); }
+
+int bbd_reproj_finalizes_itself(const bbd_reproj_args* a) { return a && reproj_launch(*a, device_facts()).finalizes_itself ? 1 : 0; }
 
 const char* bbd_reproj_kernel_name(const bbd_reproj_args* a) {
   if (!a) return "";
-  if (use_stream(a)) {
-    const bool tma = BBD_STREAM_TMA && encode_tiled() && a->width % 4 == 0 && !(((uintptr_t)a->target | (uintptr_t)a->depth | (uintptr_t)a->ident_min) & 15);
-    static char name[64];
-    if (tma && a->max_rep <= 2 && use_pipe())
-      snprintf(name, sizeof(name), "bbd::reproj_pipe_kernel<%d, %d>", a->max_rep == 1 ? 1 : 2, a->need_grad ? 1 : 0);
-    else
-      if (split_multi(a))  // selection launch <2, 0, 1> followed by the gradient launch named here
-        snprintf(name, sizeof(name), "bbd::reproj_stream%s_kernel<2, 1, 1, 1>", tma ? "_tma" : "");
-      else
-        snprintf(name, sizeof(name), "bbd::reproj_stream%s_kernel<%d, %d, %d>", tma ? "_tma" : "", a->max_rep == 1 ? 1 : 2, a->need_grad ? 1 : 0,
-                 a->max_rep > 2 ? 1 : 0);
-    return name;
-  }
-  const bool keep = StripSmem<SCfg>::floats(a->max_rep) * sizeof(float) <= 75 * 1024;
-  if (a->need_grad) return keep ? "bbd::reproj_kernel<1, 1>" : "bbd::reproj_kernel<1, 0>";
-  return keep ? "bbd::reproj_kernel<0, 1>" : "bbd::reproj_kernel<0, 0>";
+  static char name[64];
+  reproj_kernel_name(reproj_launch(*a, device_facts()), name, sizeof(name));
+  return name;
 }
 
 int bbd_reproj_finalize(const bbd_reproj_args* a, float* loss, float* gpose, bbd_stream_t stream) {
   if (!a || !loss || !a->loss_part) return fail(BBD_E_ARG, "finalize: null argument");
   if (gpose && !a->gpose_part) return fail(BBD_E_ARG, "finalize: no pose partials");
-  const int ntiles = bbd_reproj_tiles(a->height, a->width);
+  const ReprojLaunch L = reproj_launch(*a, device_facts());
   const int blocks = a->num_scales * (1 + (gpose ? a->num_pose : 0));
-  reproj_finalize_kernel<<<blocks, FIN_NT, 0, (cudaStream_t)stream>>>(*a, loss, gpose, ntiles, parts_used(a, false), parts_used(a, true));
+  reproj_finalize_kernel<<<blocks, FIN_NT, 0, (cudaStream_t)stream>>>(*a, loss, gpose, L.stride, L.used, L.used_grad);
   return check_launch("reproj_finalize_kernel");
 }
 
-static int smooth_max_parts(int levels, const int32_t* h, const int32_t* w) {
-  int mc = 1;
-  for (int l = 0; l < levels; ++l) mc = std::max(mc, std::max(sm_chunks(h[l], w[l]), smr_blocks(h[l], w[l])));
-  return mc;
-}
-// partial-sum slots (levels,B,4,parts) + the per-sample scalars (levels,B,2) + the ticket of the last-block reduction
 size_t bbd_smooth_scratch_floats(int32_t batch, int32_t levels, const int32_t* h, const int32_t* w) {
-  return (size_t)levels * batch * 4 * smooth_max_parts(levels, h, w) + (size_t)levels * batch * 2 + 4;
+  return smooth_layout(batch, levels, h, w).floats;
 }
 
 int bbd_smooth_fused(const bbd_smooth_args* in, bbd_stream_t stream) {
@@ -1005,11 +911,10 @@ int bbd_smooth_fused(const bbd_smooth_args* in, bbd_stream_t stream) {
     nby = std::max(nby, smr_nby(a.h[l]));
     total += (unsigned)(a.batch * smr_blocks(a.h[l], a.w[l]));
   }
-  const int mc = smooth_max_parts(a.levels, a.h, a.w);
-  a.max_chunks = mc;
-  float* tail = a.scratch + (size_t)a.levels * a.batch * 4 * mc;
-  float* coef = a.defer_norm ? a.coef : tail;
-  unsigned* ticket = reinterpret_cast<unsigned*>(tail + (size_t)a.levels * a.batch * 2);
+  const SmoothLayout lay = smooth_layout(a.batch, a.levels, a.h, a.w);
+  a.max_chunks = lay.max_parts;
+  float* coef = a.defer_norm ? a.coef : a.scratch + lay.scalars;
+  unsigned* ticket = reinterpret_cast<unsigned*>(a.scratch + lay.ticket);
   cudaStream_t st = (cudaStream_t)stream;
   cudaMemsetAsync(ticket, 0, sizeof(unsigned), st);
   dim3 grid(nbx, nby, a.levels * a.batch);
@@ -1077,13 +982,7 @@ int bbd_disp_to_depth_backward_pass2(const bbd_d2d_args* a, int32_t level_begin,
 
 int bbd_disp_to_depth_backward(const bbd_d2d_args* a, bbd_stream_t stream) {
   if (int rc = d2d_backward_check(a)) return rc;
-  bool fused = (((uintptr_t)a->gdepth | (uintptr_t)a->depth) & 15) == 0 && 2 * (size_t)a->width * sizeof(float) <= 48 * 1024;
-  int max_h = 1;
-  for (int l = 0; l < a->levels; ++l) {
-    fused = fused && d2d_fused_factor(*a, l) != 0;
-    max_h = std::max(max_h, a->h[l]);
-  }
-  if (fused) {  // every level in one launch, no scratch plane
+  if (d2d_single_launch(*a)) {  // every level in one launch, no scratch plane
     D2DRowList list;
     int order[BBD_MAX_SCALES];
     for (int l = 0; l < a->levels; ++l) order[l] = l;
@@ -1101,10 +1000,7 @@ int bbd_disp_to_depth_backward(const bbd_d2d_args* a, bbd_stream_t stream) {
       if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, d2d_backward_fused_kernel, threads, 2 * (size_t)a->width * sizeof(float)) != cudaSuccess || per_sm < 1) per_sm = 1;
       per_sm_threads = threads;
     }
-    int sms = 148;
-    int dev = 0;
-    if (cudaGetDevice(&dev) == cudaSuccess) cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-    const int blocks = std::min(list.begin[a->levels], sms * per_sm);
+    const int blocks = std::min(list.begin[a->levels], device_sms() * per_sm);
     d2d_backward_fused_kernel<<<blocks, threads, 2 * (size_t)a->width * sizeof(float), (cudaStream_t)stream>>>(*a, list);
     return check_launch("d2d_backward_fused_kernel");
   }

@@ -1,8 +1,9 @@
 // TEST-ONLY host harness: steps the thread-block phases of the sm_100a kernels on the CPU.
 //
 // The device kernels in baseboostdepth_b200/csrc/bbd_kernels.cu are thin drivers around the
-// __host__ __device__ phase functions of bbd_strip.cuh / bbd_smooth.cuh / bbd_ops.cuh.  This
-// file instantiates the same phase functions with g++ and runs, for every block, each
+// __host__ __device__ phase functions of bbd_strip.cuh / bbd_stream.cuh / bbd_pipe.cuh /
+// bbd_smooth.cuh / bbd_ops.cuh / bbd_framegrad.cuh.  This file instantiates the same phase
+// functions with g++ and steps the launches bbd_launch.cuh describes: for every block, each
 // phase for tid = 0..NT-1 before moving to the next (a barrier between phases), so index
 // logic, halo/reflection handling, candidate tables and the analytic gradients can be
 // checked against the oracle in the GPU-less build container.  It is never loaded by the
@@ -14,18 +15,22 @@
 
 #define BBD_EMU 1
 #include "simt.h"
-#include "../../baseboostdepth_b200/csrc/bbd_ops.cuh"
-#include "../../baseboostdepth_b200/csrc/bbd_smooth.cuh"
-#include "../../baseboostdepth_b200/csrc/bbd_strip.cuh"
-#include "../../baseboostdepth_b200/csrc/bbd_stream.cuh"
+#include "../../baseboostdepth_b200/csrc/bbd_launch.cuh"
 #include "../../baseboostdepth_b200/csrc/bbd_pipe.cuh"
+#include "../../baseboostdepth_b200/csrc/bbd_framegrad.cuh"
 
 using namespace bbd;
-#ifndef BBD_TILE_H
-#define BBD_TILE_H 16
-#endif
-using SCfg = StripCfg<BBD_TILE_H, 6>;
 #define FOR_STID for (int tid = 0; tid < SCfg::NT; ++tid)
+
+// The launch decisions (bbd_launch.cuh) are taken for a B200: 148 SMs and a tensor-map encoder
+// (-DBBD_EMU_NO_TMA steps the plain-load kernels instead).
+static LaunchDevice b200() {
+#ifdef BBD_EMU_NO_TMA
+  return {148, false, pipe_requested()};
+#else
+  return {148, true, pipe_requested()};
+#endif
+}
 
 extern "C" {
 
@@ -44,37 +49,7 @@ long emu_div_const_mismatches(float d) {
   return bad;
 }
 
-static int tile_parts(int height, int width) {
-  return ((width + SCfg::TW - 1) / SCfg::TW) * ((height + SCfg::TH - 1) / SCfg::TH);
-}
-int emu_reproj_tiles(int32_t height, int32_t width) {
-  int a = tile_parts(height, width);
-  if (StreamGeo::strips(width) * stream_max_segs(height) > a) a = StreamGeo::strips(width) * stream_max_segs(height);
-  if (StreamGeoM::units(height, width) > a) a = StreamGeoM::units(height, width);
-  return a;
-}
-// same choice as the launcher in bbd_kernels.cu
-static bool use_stream(const bbd_reproj_args* a) {
-  if (a->force_tile || a->min_rep < 1 || a->max_rep > BBD_MAX_REP) return false;
-  if (BBD_STREAM_ASYNC && a->max_rep > 2) return false;
-  bool any = false;
-  for (int f = 0; f < BBD_MAX_FRAMES; ++f) {
-    if (a->frames[f] && !a->frames_rgba[f]) return false;
-    any = any || a->frames_rgba[f];
-  }
-  return any;
-}
-// same choices as the launcher in bbd_kernels.cu
-static bool split_multi(const bbd_reproj_args* a) {
-  return use_stream(a) && a->max_rep > 2 && a->need_grad && a->winner != nullptr;
-}
-static int parts_used(const bbd_reproj_args* a, bool grad_parts) {
-  if (!use_stream(a)) return tile_parts(a->height, a->width);
-  if (a->max_rep > 2 && !(grad_parts && split_multi(a))) return StreamGeoM::units(a->height, a->width);
-  const int rh = a->max_rep > 2 ? stream_seg_rows_uneven(a->height, a->width, a->num_scales * a->batch, 148 * 8)
-                                : stream_seg_rows(a->height, a->width, a->num_scales * a->batch, 148 * 8);
-  return StreamGeo::strips(a->width) * ((a->height + rh - 1) / rh);
-}
+int emu_reproj_tiles(int32_t height, int32_t width) { return reproj_slots(height, width); }
 
 int emu_project_coords(int32_t n, int32_t H, int32_t W, const float* depth, const float* inv_K, const float* P, float* grid,
                        float* pix) {
@@ -99,48 +74,28 @@ int emu_pack_rgba(int32_t n, int32_t H, int32_t W, const float* planar, float* r
 }
 
 }  // extern "C"
-template <int K, bool GRAD, bool MULTI, bool WING = false>
-static void emu_stream(const bbd_reproj_args& a) {
-  const int n_units = a.num_scales * a.batch * parts_used(&a, WING);
-  const int stride = emu_reproj_tiles(a.height, a.width);
-  // like the launcher: the TMA-staged variant when the planes can be described to the TMA unit
-#ifdef BBD_EMU_NO_TMA
-  const bool tma = false;
-#else
-  const bool tma = !BBD_STREAM_ASYNC && a.width % 4 == 0;
-#endif
+// one launch of the streaming or pipelined form: every unit (warp, or block of the pipelined form) in turn
+template <int K, bool GRAD, bool MULTI, bool WING>
+static void emu_stream(const bbd_reproj_args& a, const ReprojLaunch& L, const KernelLaunch& l) {
   std::vector<float> smem(StreamSmem<K, true, MULTI>::FLOATS + StreamSmem<K, false, MULTI>::FLOATS + PipeSmem<K, GRAD>::FLOATS);
   StreamTmaMaps none = {nullptr, nullptr, nullptr};
-  const int seg_rows = (MULTI && !WING) ? BBD_STREAM_RHM
-                       : (MULTI ? stream_seg_rows_uneven(a.height, a.width, a.num_scales * a.batch, 148 * 8)
-                                : stream_seg_rows(a.height, a.width, a.num_scales * a.batch, 148 * 8));
-  // like the launcher: the pipelined three-warp form for single-sweep launches when BBD_PIPE=1
-  const char* pe = getenv("BBD_PIPE");
-  const bool pipe = tma && !MULTI && (pe ? pe[0] != '0' : false);
-  for (int unit = 0; unit < n_units; ++unit) {
-#if !BBD_STREAM_ASYNC
-    if (pipe) {
-      simt::run_block(GRAD ? 96 : 64, [&](int tid) { pipe_unit<K, GRAD>(a, unit, tid, smem.data(), stride, none, seg_rows); });
-      continue;
-    }
-    if (tma) {
-      simt::run_block(32, [&](int tid) { stream_unit<K, GRAD, true, MULTI, WING>(a, unit, tid, smem.data(), stride, none, seg_rows); });
-      continue;
-    }
-#endif
-    simt::run_block(32, [&](int tid) { stream_unit<K, GRAD, false, MULTI, WING>(a, unit, tid, smem.data(), stride, none, seg_rows); });
+  for (int unit = 0; unit < l.units; ++unit) {
+    if (L.form == REPROJ_PIPE)
+      simt::run_block(GRAD ? 96 : 64, [&](int tid) { pipe_unit<K, GRAD>(a, unit, tid, smem.data(), L.stride, none, l.seg_rows); });
+    else if (L.tma)
+      simt::run_block(32, [&](int tid) { stream_unit<K, GRAD, true, MULTI, WING>(a, unit, tid, smem.data(), L.stride, none, l.seg_rows); });
+    else
+      simt::run_block(32, [&](int tid) { stream_unit<K, GRAD, false, MULTI, WING>(a, unit, tid, smem.data(), L.stride, none, l.seg_rows); });
   }
-  (void)tma;
 }
 extern "C" {
 
 int emu_ident_forward(const bbd_ident_args* ap) {
   const bbd_ident_args& a = *ap;
-  if (!a.force_tile) {
-    const int seg_rows = ident_seg_rows(a.height, a.width, a.batch, 148 * 16);
-    const int n_units = a.batch * IdentGeo::strips(a.width) * ((a.height + seg_rows - 1) / seg_rows);
-    for (int unit = 0; unit < n_units; ++unit)
-      simt::run_block(32, [&](int tid) { ident_unit(a, const_cast<float* const*>(a.frames_rgba), unit, tid, seg_rows); });
+  const IdentLaunch L = ident_launch(a, b200().sms);
+  if (L.stream) {
+    for (int unit = 0; unit < L.units; ++unit)
+      simt::run_block(32, [&](int tid) { ident_unit(a, const_cast<float* const*>(a.frames_rgba), unit, tid, L.seg_rows); });
     return 0;
   }
   std::vector<float> smem(IdentStripSmem<SCfg>::floats());
@@ -171,19 +126,16 @@ int emu_ident_forward(const bbd_ident_args* ap) {
 
 int emu_reproj_fused(const bbd_reproj_args* ap) {
   const bbd_reproj_args& a = *ap;
-  if (use_stream(ap)) {
-    if (a.max_rep == 1) { if (a.need_grad) emu_stream<1, true, false>(a); else emu_stream<1, false, false>(a); }
-    else if (a.max_rep == 2) { if (a.need_grad) emu_stream<2, true, false>(a); else emu_stream<2, false, false>(a); }
-#if !BBD_STREAM_ASYNC
-    else if (split_multi(&a)) { emu_stream<2, false, true>(a); emu_stream<2, true, true, true>(a); }
-    else { if (a.need_grad) emu_stream<2, true, true>(a); else emu_stream<2, false, true>(a); }
-#endif
+  const ReprojLaunch L = reproj_launch(a, b200());
+  if (L.form != REPROJ_TILE) {
+    for (int i = 0; i < L.n_launches; ++i)
+      with_stream_instance(L, L.launch[i], [&](auto k, auto grad, auto multi, auto wing) {
+        emu_stream<decltype(k)::value, decltype(grad)::value, decltype(multi)::value, decltype(wing)::value>(a, L, L.launch[i]);
+      });
     return 0;
   }
-  // the CPU harness runs the reuse (non-KEEP) variant for batches with more than two candidates,
-  // like the launcher does
-  const bool keep = StripSmem<SCfg>::floats(a.max_rep) * sizeof(float) <= 75 * 1024;
-  std::vector<float> smem(StripSmem<SCfg>::floats(keep ? a.max_rep : 1));
+  const bool keep = L.keep;
+  std::vector<float> smem(L.tile_smem / sizeof(float));
   std::vector<float> red(12 * SCfg::NT + 12 * SCfg::RED_SEG * 2);  // host-side reduction scratch
   std::vector<float> gPs((size_t)SCfg::NT * 12), parts(SCfg::NT);
   std::vector<StripCtx> ctx(SCfg::NT);
@@ -244,14 +196,18 @@ int emu_reproj_fused(const bbd_reproj_args* ap) {
   return 0;
 }
 
-const char* emu_reproj_kernel_name(const bbd_reproj_args*) { return "emulation"; }
-int emu_reproj_finalizes_itself(const bbd_reproj_args* a) {
-  return a && use_stream(a) && a->max_rep <= 2 && a->tickets && a->pair_sum && a->loss_out && (!a->need_grad || a->gpose_out) ? 1 : 0;
+const char* emu_reproj_kernel_name(const bbd_reproj_args* a) {
+  if (!a) return "";
+  static char name[64];
+  reproj_kernel_name(reproj_launch(*a, b200()), name, sizeof(name));
+  return name;
 }
+int emu_reproj_finalizes_itself(const bbd_reproj_args* a) { return a && reproj_launch(*a, b200()).finalizes_itself ? 1 : 0; }
 
 int emu_reproj_finalize(const bbd_reproj_args* ap, float* loss, float* gpose) {
   const bbd_reproj_args& a = *ap;
-  const int ntiles = emu_reproj_tiles(a.height, a.width), used = parts_used(ap, false), used_grad = parts_used(ap, true);
+  const ReprojLaunch L = reproj_launch(a, b200());
+  const int ntiles = L.stride, used = L.used, used_grad = L.used_grad;
   for (int s = 0; s < a.num_scales; ++s) {
     float tot = 0.0f;
     for (int i = 0; i < a.batch * used; ++i) tot += a.loss_part[(size_t)s * a.batch * ntiles + (size_t)(i / used) * ntiles + (i % used)];
@@ -275,24 +231,15 @@ int emu_reproj_finalize(const bbd_reproj_args* ap, float* loss, float* gpose) {
   return 0;
 }
 
-static int smooth_max_parts(int levels, const int32_t* h, const int32_t* w) {
-  int mc = 1;
-  for (int l = 0; l < levels; ++l) {
-    const int c = sm_chunks(h[l], w[l]) > smr_blocks(h[l], w[l]) ? sm_chunks(h[l], w[l]) : smr_blocks(h[l], w[l]);
-    mc = c > mc ? c : mc;
-  }
-  return mc;
-}
 size_t emu_smooth_scratch_floats(int32_t batch, int32_t levels, const int32_t* h, const int32_t* w) {
-  return (size_t)levels * batch * 4 * smooth_max_parts(levels, h, w) + (size_t)levels * batch * 2 + 4;
+  return smooth_layout(batch, levels, h, w).floats;
 }
 
 int emu_smooth_fused(const bbd_smooth_args* in) {
   bbd_smooth_args a = *in;
-  const int mc = smooth_max_parts(a.levels, a.h, a.w);
-  a.max_chunks = mc;
-  float* tail = a.scratch + (size_t)a.levels * a.batch * 4 * mc;
-  float* coef = a.defer_norm ? a.coef : tail;
+  const SmoothLayout lay = smooth_layout(a.batch, a.levels, a.h, a.w);
+  a.max_chunks = lay.max_parts;
+  float* coef = a.defer_norm ? a.coef : a.scratch + lay.scalars;
   // stage 2: one fiber block per warp of the device kernel's blocks
   for (int lvl = 0; lvl < a.levels; ++lvl)
     for (int b = 0; b < a.batch; ++b) {
@@ -383,9 +330,7 @@ static void emu_d2d_fused_level(const bbd_d2d_args& a, int lvl) {
 extern "C" {
 int emu_disp_to_depth_backward(const bbd_d2d_args* ap) {
   const bbd_d2d_args& a = *ap;
-  bool fused = true;  // same choice as the launcher
-  for (int l = 0; l < a.levels; ++l) fused = fused && d2d_fused_factor(a, l) != 0;
-  if (fused) {
+  if (d2d_single_launch(a)) {
     for (int l = 0; l < a.levels; ++l) {
       const int f = d2d_fused_factor(a, l);
       if (f == 1) emu_d2d_fused_level<1>(a, l);
@@ -508,6 +453,51 @@ int emu_loss_combine_backward(int32_t n, const float* g_total, const float* g_pe
 
 int emu_u8_to_f32(const uint8_t* src, float* dst, size_t n) {
   for (size_t i = 0; i < n; ++i) dst[i] = u8_to_unit(src[i]);
+  return 0;
+}
+
+// gradients w.r.t. the colour frames (bbd_framegrad.cuh), one pixel at a time
+int emu_frame_grad(const bbd_reproj_args* ap, const bbd_frame_grad_args* fp) {
+  const bbd_reproj_args& a = *ap;
+  const bbd_frame_grad_args& f = *fp;
+  const int H = a.height, W = a.width;
+  if (!a.no_ssim)
+    for (int sb = 0; sb < a.num_scales * a.batch; ++sb)
+      for (int q = 0; q < H * W; ++q) fg_coef_px(a, f, sb / a.batch, sb % a.batch, q / W, q % W);
+  for (int b = 0; b < a.batch; ++b)
+    for (int p = 0; p < H * W; ++p) fg_pred_px(a, f, b, p / W, p % W);
+  return 0;
+}
+
+int emu_frame_grad_stacks(const bbd_reproj_args* ap, const bbd_frame_grad_args* fp) {
+  const bbd_reproj_args& a = *ap;
+  const bbd_frame_grad_args& f = *fp;
+  const int HW = a.height * a.width, rows = fg_total_rows(f);
+  if (!rows) return 0;
+  const int n_items = a.num_scales * a.batch * a.max_rep * HW, n_keys = rows * HW;
+  for (int i = 0; i <= n_items; ++i) gs_segment_mark(f.keys_sorted, n_items, n_keys, i, f.seg_start);
+  for (int grow = 0; grow < rows; ++grow) {
+    int slot, row;
+    fg_locate_row(f, grow, slot, row);
+    if (!f.gframes[slot]) continue;
+    for (int c = 0; c < 3; ++c)
+      for (int p = 0; p < HW; ++p) f.gframes[slot][((size_t)row * 3 + c) * HW + p] = fg_stack_px(a, f, slot, row, c, p);
+  }
+  return 0;
+}
+
+int emu_smooth_image_grad(const bbd_smooth_img_args* ap) {
+  const bbd_smooth_img_args& a = *ap;
+  for (int lvl = 0; lvl < a.levels; ++lvl) {
+    if (!a.gimg[lvl]) continue;
+    const int n = a.h[lvl] * a.w[lvl];
+    for (int b = 0; b < a.batch; ++b)
+      for (int i = 0; i < n; ++i) {
+        float g[3];
+        smi_px(a, lvl, b, i / a.w[lvl], i % a.w[lvl], g);
+        for (int c = 0; c < 3; ++c) a.gimg[lvl][((size_t)b * 3 + c) * n + i] = g[c];
+      }
+  }
   return 0;
 }
 

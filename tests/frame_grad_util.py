@@ -1,36 +1,7 @@
-"""Test plumbing of the colour-frame gradients: the CPU harness with the frame-gradient entry points, and
-helpers that mark, read and check the gradients of a batch's colour tensors."""
+"""Test helpers of the colour-frame gradients: mark, read and check the gradients of a batch's colour tensors."""
 from __future__ import annotations
 
-import os
-import subprocess
-import tempfile
-
 import torch
-
-from baseboostdepth_b200 import _lib
-from fused_util import EMU_DIR
-
-_EMU = None
-
-
-def emu_frame_backend() -> _lib.Backend:
-    """Compile (if stale) and load the CPU harness of tests/emu/bbd_emu.cpp together with the emu_* versions of
-    the frame-gradient entry points (tests/emu/bbd_emu_framegrad.cpp).  Built next to the sources, or in the
-    temporary directory when the tree is read-only."""
-    global _EMU
-    if _EMU is None:
-        src = os.path.join(EMU_DIR, "bbd_emu_framegrad.cpp")
-        out_dir = EMU_DIR if os.access(EMU_DIR, os.W_OK) else tempfile.gettempdir()
-        so = os.path.join(out_dir, "libbbd_emu_framegrad.so")
-        csrc = os.path.join(os.path.dirname(EMU_DIR), "..", "baseboostdepth_b200", "csrc")
-        deps = [src, os.path.join(EMU_DIR, "bbd_emu.cpp"), os.path.join(EMU_DIR, "simt.h")] + [
-            os.path.join(csrc, f) for f in os.listdir(csrc)]
-        if not os.path.exists(so) or any(os.path.getmtime(d) > os.path.getmtime(so) for d in deps):
-            subprocess.run(["g++", "-O2", "-std=c++17", "-ffp-contract=off", "-mfma", "-shared", "-fPIC", "-o", so, src],
-                           check=True)
-        _EMU = _lib.Backend(so, "emu_", cuda=False)
-    return _EMU
 
 
 def frame_keys(inputs):

@@ -3,6 +3,7 @@ from __future__ import annotations
 
 import os
 import subprocess
+import tempfile
 
 import torch
 
@@ -15,14 +16,16 @@ _EMU = None
 
 def emu_backend(flags: str = None) -> _lib.Backend:
     """Compile (if stale) and load tests/emu/libbbd_emu*.so -- the kernels' phase code run on the CPU.
-    ``flags`` (or $BBD_EMU_FLAGS): extra -D options selecting a kernel variant, built into its own file."""
+    ``flags`` (or $BBD_EMU_FLAGS): extra -D options selecting a kernel variant, built into its own file.
+    Built next to the sources, or in the temporary directory when the tree is read-only."""
     global _EMU
     flags = os.environ.get("BBD_EMU_FLAGS", "") if flags is None else flags
     if _EMU is None:
         _EMU = {}
     if flags not in _EMU:
         tag = "".join(ch if ch.isalnum() else "_" for ch in flags)
-        so, src = os.path.join(EMU_DIR, f"libbbd_emu{tag}.so"), os.path.join(EMU_DIR, "bbd_emu.cpp")
+        out_dir = EMU_DIR if os.access(EMU_DIR, os.W_OK) else tempfile.gettempdir()
+        so, src = os.path.join(out_dir, f"libbbd_emu{tag}.so"), os.path.join(EMU_DIR, "bbd_emu.cpp")
         csrc = os.path.join(os.path.dirname(EMU_DIR), "..", "baseboostdepth_b200", "csrc")
         deps = [src, os.path.join(EMU_DIR, "simt.h")] + [os.path.join(csrc, f) for f in os.listdir(csrc)]
         if not os.path.exists(so) or any(os.path.getmtime(d) > os.path.getmtime(so) for d in deps):

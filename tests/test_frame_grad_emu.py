@@ -13,8 +13,8 @@ import torch
 
 from baseboostdepth_b200 import _lib
 from baseboostdepth_b200 import layers as L
-from frame_grad_util import emu_frame_backend, frame_grad, frame_keys, referenced_rows, require_frame_grads
-from fused_util import run_fused
+from frame_grad_util import frame_grad, frame_keys, referenced_rows, require_frame_grads
+from fused_util import emu_backend, run_fused
 from helpers import Golden, assert_grad_parity, golden_cases, rel_l2
 from oracle import loss_path as O
 
@@ -36,7 +36,7 @@ def _fused(case, keys, groups, detach_params=False, backend=None):
         for k, v in list(h.outputs.items()):
             h.outputs[k] = v.detach()
     require_frame_grads(h.inputs, keys)
-    losses, plan = run_fused(h.inputs, h.outputs, h.opt(), h.noise, h.num_scales, backend=backend or emu_frame_backend(),
+    losses, plan = run_fused(h.inputs, h.outputs, h.opt(), h.noise, h.num_scales, backend=backend or emu_backend(),
                              groups=groups)
     losses["loss"].backward()
     return h, losses, plan
@@ -72,7 +72,7 @@ def test_frame_grads_match_oracle(case):
     g0 = Golden(case)
     ref, aux = O.run(g0.inputs, g0.outputs, g0.opt(), g0.noise, num_scales=g0.num_scales)
     n = Golden(case)
-    losses0, _ = run_fused(n.inputs, n.outputs, n.opt(), n.noise, n.num_scales, backend=emu_frame_backend(), groups=aux["groups"])
+    losses0, _ = run_fused(n.inputs, n.outputs, n.opt(), n.noise, n.num_scales, backend=emu_backend(), groups=aux["groups"])
     losses0["loss"].backward()
     for k in losses0:
         assert torch.equal(losses0[k].detach(), losses[k].detach()), k
@@ -131,7 +131,7 @@ def test_default_step_makes_the_same_calls(case, finalize):
     """A step whose frames need no gradient makes exactly the calls it made before frame gradients existed
     (the fused finalize of the one/two-candidate streaming kernel saves reproj_finalize)."""
     g = Golden(case)
-    rec = _Recorder(emu_frame_backend())
+    rec = _Recorder(emu_backend())
     losses, _ = run_fused(g.inputs, g.outputs, g.opt(), g.noise, g.num_scales, backend=rec)
     losses["loss"].backward()
     assert rec.names == ["disp_to_depth_forward", "smooth_fused", "pose_pack_forward", "ident_forward",
@@ -139,7 +139,7 @@ def test_default_step_makes_the_same_calls(case, finalize):
                                                        "disp_to_depth_backward", "pose_pack_backward"], rec.names
     h = Golden(case)
     require_frame_grads(h.inputs)
-    rec = _Recorder(emu_frame_backend())
+    rec = _Recorder(emu_backend())
     losses, _ = run_fused(h.inputs, h.outputs, h.opt(), h.noise, h.num_scales, backend=rec)
     losses["loss"].backward()
     assert NEW_CALLS <= set(rec.names)
@@ -147,7 +147,7 @@ def test_default_step_makes_the_same_calls(case, finalize):
 
 @pytest.mark.parametrize("shape", [(2, 3, 10, 14), (1, 3, 7, 2), (3, 3, 2, 9), (2, 3, 13, 11)])
 def test_tier_a_smooth_loss_image_gradient(shape, monkeypatch):
-    monkeypatch.setattr(L, "_TEST_BACKEND", emu_frame_backend())
+    monkeypatch.setattr(L, "_TEST_BACKEND", emu_backend())
     gen = torch.Generator().manual_seed(17)
     n, c, h, w = shape
     disp0 = torch.rand(n, 1, h, w, generator=gen)
