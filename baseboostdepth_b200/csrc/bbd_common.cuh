@@ -12,6 +12,7 @@
 // 4-tap accumulation.  The helpers below therefore use the explicitly rounded
 // intrinsics (never contracted by nvcc) and FMA only where the reference has it.
 #pragma once
+#include <assert.h>
 #include <math.h>
 #include <stdint.h>
 
@@ -93,6 +94,7 @@ BBD_HD f4 load4(const float* p) {
   f4 r; r.x = v.x; r.y = v.y; r.z = v.z; r.w = v.w;
   return r;
 #else
+  assert(((uintptr_t)p & 15) == 0 && "load4: a 16-byte load needs a 16-byte aligned address");
   f4 r; r.x = p[0]; r.y = p[1]; r.z = p[2]; r.w = p[3];
   return r;
 #endif

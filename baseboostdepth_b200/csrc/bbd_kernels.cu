@@ -384,7 +384,7 @@ __global__ void __launch_bounds__(256) smooth_apply_kernel(const SmoothArgs a, c
 // the row taps.
 // grid (column blocks, row groups, levels): a thread owns four consecutive columns, whose source
 // taps it computes once, and walks rows (b, py); no per-thread division, float4 stores.
-__global__ void __launch_bounds__(128) d2d_forward_kernel(const bbd_d2d_args a) {
+__global__ void __launch_bounds__(128) d2d_forward_kernel(const bbd_d2d_args a, const bool vec) {
   const int lvl = blockIdx.z;
   const int H = a.height, W = a.width, HW = H * W;
   const int h = a.h[lvl], w = a.w[lvl];
@@ -392,8 +392,7 @@ __global__ void __launch_bounds__(128) d2d_forward_kernel(const bbd_d2d_args a) 
   const int g = blockIdx.x * blockDim.x + threadIdx.x;
   if (g >= gw) return;
   const float sy = div_((float)h, (float)H), sx = div_((float)w, (float)W);
-  float* out = a.depth + (size_t)lvl * a.batch * HW;
-  const bool vec = (W % 4) == 0;
+  float* out = a.depth + (size_t)lvl * a.batch * HW;  // vec: d2d_forward_vec (bbd_launch.cuh)
   const bool same = (h == H && w == W);  // taps are (o, o) with weights (1, 0): the value itself
   Lerp tx[4];
 #pragma unroll
@@ -815,6 +814,7 @@ const char* bbd_last_error_string(void) { return g_err; }
 int bbd_ident_forward(const bbd_ident_args* a, bbd_stream_t stream) {
   if (!a || !a->target || !a->ident_min || !a->tab.hdr || !a->tab.ident) return fail(BBD_E_ARG, "ident: null argument");
   if (a->batch <= 0 || a->height < 2 || a->width < 2) return fail(BBD_E_ARG, "ident: bad size");
+  if (!rgba_aligned(a->frames_rgba)) return fail(BBD_E_ARG, "ident: frames_rgba entries must be 16-byte aligned");
   const IdentLaunch L = ident_launch(*a, device_sms());
   if (L.stream) {
     RgbaPtrs rp;
@@ -840,6 +840,7 @@ int bbd_reproj_fused(const bbd_reproj_args* a, bbd_stream_t stream) {
   if (a->need_grad && (!a->gpose_part || !a->gdepth)) return fail(BBD_E_ARG, "reproj: gradient buffers missing");
   if (a->batch <= 0 || a->height < 2 || a->width < 2 || a->num_scales <= 0) return fail(BBD_E_ARG, "reproj: bad size");
   if (a->max_rep < 1 || a->max_rep > BBD_MAX_REP) return fail(BBD_E_RANGE, "reproj: max_rep out of range");
+  if (!rgba_aligned(a->frames_rgba)) return fail(BBD_E_ARG, "reproj: frames_rgba entries must be 16-byte aligned");
   const ReprojLaunch L = reproj_launch(*a, device_facts());
   if (a->tickets && !L.finalizes_itself) return fail(BBD_E_ARG, "reproj: tickets given but pair_sum / loss_out / gpose_out missing or tile kernel selected");
   if (L.form != REPROJ_TILE) {
@@ -937,7 +938,7 @@ int bbd_disp_to_depth_forward(const bbd_d2d_args* a, bbd_stream_t stream) {
     if (!a->disp[l] || a->h[l] < 1 || a->w[l] < 1) return fail(BBD_E_ARG, "d2d forward: bad level");
   const size_t rows = (size_t)a->batch * a->height;
   dim3 grid((unsigned)(((a->width + 3) / 4 + 127) / 128), (unsigned)std::min<size_t>(rows, kRowBlocks), a->levels);
-  d2d_forward_kernel<<<grid, 128, 0, (cudaStream_t)stream>>>(*a);
+  d2d_forward_kernel<<<grid, 128, 0, (cudaStream_t)stream>>>(*a, d2d_forward_vec(*a));
   return check_launch("d2d_forward_kernel");
 }
 
@@ -1139,9 +1140,10 @@ int bbd_project_coords(int32_t n, int32_t height, int32_t width, const float* de
 
 int bbd_pack_rgba(int32_t n, int32_t height, int32_t width, const float* planar, float* rgba, bbd_stream_t stream) {
   if (!planar || !rgba) return fail(BBD_E_ARG, "pack_rgba: null argument");
+  if (!aligned16(rgba)) return fail(BBD_E_ARG, "pack_rgba: rgba must be 16-byte aligned");  // one float4 per pixel
   if (n <= 0) return 0;
   const int HW = height * width;
-  const bool vec = (HW % 4 == 0) && ((uintptr_t)planar % 16 == 0) && ((uintptr_t)rgba % 16 == 0);
+  const bool vec = (HW % 4 == 0) && aligned16(planar);
   if (vec)
     pack_rgba_kernel<<<grid_for((size_t)n * HW / 4, 256), 256, 0, (cudaStream_t)stream>>>(n, HW, planar, reinterpret_cast<float4*>(rgba));
   else

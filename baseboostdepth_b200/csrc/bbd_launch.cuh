@@ -56,6 +56,24 @@ inline bool pipe_requested() {
   return e ? (e[0] != '0') : (BBD_USE_PIPE != 0);
 }
 
+// ---- alignment of caller-supplied buffers --------------------------------------------------------
+// A 16-byte access (float4 / LDG.128 / STG.128, a TMA box) to a buffer the caller owns is issued only where the
+// buffer's address allows it; every such access is decided here.
+inline bool aligned16(const void* p) { return ((uintptr_t)p & 15) == 0; }
+
+// The channel-interleaved frame copies (frames_rgba) are written and read one 16-byte pixel at a time, in every
+// form: bbd_pack_rgba, bbd_ident_forward and bbd_reproj_fused reject a non-NULL entry that is not 16-byte aligned.
+template <class T>
+inline bool rgba_aligned(T* const* rgba) {
+  for (int f = 0; f < BBD_MAX_FRAMES; ++f)
+    if (!aligned16(rgba[f])) return false;
+  return true;
+}
+
+// disp_to_depth forward: a thread stores its four pixels as one float4 when rows are whole float4s and the depth
+// planes start on a 16-byte boundary; otherwise four scalar stores.
+inline bool d2d_forward_vec(const bbd_d2d_args& a) { return a.width % 4 == 0 && aligned16(a.depth); }
+
 // ---- fused reprojection loss ------------------------------------------------------------------
 enum ReprojForm { REPROJ_TILE, REPROJ_STREAM, REPROJ_PIPE };
 
@@ -115,8 +133,7 @@ inline ReprojLaunch reproj_launch(const bbd_reproj_args& a, const LaunchDevice& 
     return L;
   }
   // widths that are not a multiple of four floats (or unaligned planes) cannot be described to the TMA unit
-  L.tma = BBD_STREAM_TMA && dev.tma && a.width % 4 == 0 &&
-          !(((uintptr_t)a.target | (uintptr_t)a.depth | (uintptr_t)a.ident_min) & 15);
+  L.tma = BBD_STREAM_TMA && dev.tma && a.width % 4 == 0 && aligned16(a.target) && aligned16(a.depth) && aligned16(a.ident_min);
   L.k = a.max_rep == 1 ? 1 : 2;
   const bool multi = a.max_rep > 2;
   L.form = L.tma && !multi && dev.pipe ? REPROJ_PIPE : REPROJ_STREAM;
@@ -211,10 +228,15 @@ inline SmoothLayout smooth_layout(int batch, int levels, const int32_t* h, const
 
 // ---- disparity backward -------------------------------------------------------------------------
 // Every level in one launch (no scratch plane) when each has a supported factor and two full-resolution rows of
-// tent sums fit the shared memory; otherwise the two-pass form.
+// tent sums fit the shared memory; otherwise the two-pass form.  The single launch reads gdepth and depth 16 bytes
+// at a time and stores the gradient of a full-resolution (factor 1) level as float4s: those buffers must be 16-byte
+// aligned.  (It reads gsmooth one element at a time.)
 inline bool d2d_single_launch(const bbd_d2d_args& a) {
-  bool fused = (((uintptr_t)a.gdepth | (uintptr_t)a.depth) & 15) == 0 && 2 * (size_t)a.width * sizeof(float) <= 48 * 1024;
-  for (int l = 0; l < a.levels; ++l) fused = fused && d2d_fused_factor(a, l) != 0;
+  bool fused = aligned16(a.gdepth) && aligned16(a.depth) && 2 * (size_t)a.width * sizeof(float) <= 48 * 1024;
+  for (int l = 0; l < a.levels; ++l) {
+    const int f = d2d_fused_factor(a, l);
+    fused = fused && f != 0 && (f != 1 || aligned16(a.gdisp[l]));
+  }
   return fused;
 }
 

@@ -24,6 +24,14 @@
  *   - Return value: 0 on success, a cudaError_t (>0) if a launch failed, or a
  *     negative BBD_E_* code for a bad argument.  Nothing throws, nothing exits.
  *   - There is no CPU implementation behind these symbols.
+ *   - Alignment: every pointer must be aligned to its element type (4 bytes for float and int32).  Where a
+ *     kernel can move 16 bytes at a time it checks the pointer first and falls back to narrower accesses when
+ *     the address is not 16-byte aligned (the fused loss's TMA staging of target / depth / ident_min, the
+ *     disparity -> depth forward's depth stores, the single-launch disparity backward's gdepth / depth loads and
+ *     full-resolution gdisp stores, bbd_pack_rgba's planar loads, bbd_u8_to_f32).  The one exception is the
+ *     channel-interleaved frame copies (frames_rgba, the rgba output of bbd_pack_rgba), which are only ever
+ *     accessed one 16-byte pixel at a time: a non-NULL entry that is not 16-byte aligned is rejected with
+ *     BBD_E_ARG.  Buffers from cudaMalloc or the PyTorch allocator always satisfy this.
  */
 #ifndef BBD_LOSS_H_
 #define BBD_LOSS_H_
@@ -76,7 +84,7 @@ typedef struct bbd_ident_args {
   uint8_t* ident_arg;
   /* Optional: (n_f,H,W,4) channel-interleaved copies of the frame stacks, written as a by-product (every
    * source row passes through registers here anyway); the layout bbd_reproj_args.frames_rgba expects.
-   * NULL entries are skipped. */
+   * NULL entries are skipped; a non-NULL entry must be 16-byte aligned (BBD_E_ARG otherwise). */
   float* frames_rgba[BBD_MAX_FRAMES];
   int32_t force_tile; /* 0: streaming form (contracted / separable arithmetic); != 0: tile kernel with the
                          reference's rounding, no copies written */
@@ -114,7 +122,8 @@ typedef struct bbd_reproj_args {
   /* Optional channel-interleaved copies of the frame stacks, (n_f,H,W,4) = r,g,b,0 per pixel, written by
    * bbd_pack_rgba: one 16-byte load fetches a bilinear tap of all three channels.  When every stack
    * that the tables reference has one, and 1 <= min_rep <= max_rep <= 2, bbd_reproj_fused runs the
-   * streaming kernel (csrc/bbd_stream.cuh); otherwise the tile kernel, which reads `frames`. */
+   * streaming kernel (csrc/bbd_stream.cuh); otherwise the tile kernel, which reads `frames`.  Every non-NULL
+   * entry must be 16-byte aligned (BBD_E_ARG otherwise). */
   const float* frames_rgba[BBD_MAX_FRAMES];
   int32_t min_rep;    /* min n_rep over the batch (0 = unknown: tile kernel) */
   /* Optional fused finalize (streaming kernel only; see bbd_reproj_finalizes_itself): when `tickets` is set the
@@ -135,7 +144,8 @@ int bbd_reproj_tiles(int32_t height, int32_t width); /* partial-sum slots per (s
  * is the north-west bilinear tap.  Either output may be NULL. */
 int bbd_project_coords(int32_t n, int32_t height, int32_t width, const float* depth, const float* inv_K, const float* P,
                        float* grid, float* pix, bbd_stream_t stream);
-/* (n,3,H,W) planar -> (n,H,W,4) interleaved, 4th component 0: the gather layout of the streaming kernel. */
+/* (n,3,H,W) planar -> (n,H,W,4) interleaved, 4th component 0: the gather layout of the streaming kernel.
+ * rgba must be 16-byte aligned (BBD_E_ARG otherwise); planar may start anywhere. */
 int bbd_pack_rgba(int32_t n, int32_t height, int32_t width, const float* planar, float* rgba, bbd_stream_t stream);
 int bbd_reproj_fused(const bbd_reproj_args* a, bbd_stream_t stream);
 /* 1 if bbd_reproj_fused, for these arguments, also performs the reduction of bbd_reproj_finalize (tickets given

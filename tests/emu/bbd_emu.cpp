@@ -92,6 +92,7 @@ extern "C" {
 
 int emu_ident_forward(const bbd_ident_args* ap) {
   const bbd_ident_args& a = *ap;
+  if (!rgba_aligned(a.frames_rgba)) return BBD_E_ARG;
   const IdentLaunch L = ident_launch(a, b200().sms);
   if (L.stream) {
     for (int unit = 0; unit < L.units; ++unit)
@@ -126,6 +127,7 @@ int emu_ident_forward(const bbd_ident_args* ap) {
 
 int emu_reproj_fused(const bbd_reproj_args* ap) {
   const bbd_reproj_args& a = *ap;
+  if (!rgba_aligned(a.frames_rgba)) return BBD_E_ARG;
   const ReprojLaunch L = reproj_launch(a, b200());
   if (L.form != REPROJ_TILE) {
     for (int i = 0; i < L.n_launches; ++i)
@@ -275,14 +277,22 @@ int emu_smooth_fused(const bbd_smooth_args* in) {
   return 0;
 }
 
+// four pixels of a row per thread, stored as the device kernel stores them (one float4 where d2d_forward_vec allows)
 int emu_disp_to_depth_forward(const bbd_d2d_args* ap) {
   const bbd_d2d_args& a = *ap;
-  const int HW = a.height * a.width;
+  const int H = a.height, W = a.width;
+  const bool vec = d2d_forward_vec(a);
   for (int lvl = 0; lvl < a.levels; ++lvl) {
-    const float sy = (float)a.h[lvl] / (float)a.height, sx = (float)a.w[lvl] / (float)a.width;
-    for (int b = 0; b < a.batch; ++b)
-      for (int i = 0; i < HW; ++i)
-        a.depth[((size_t)lvl * a.batch + b) * HW + i] = d2d_forward_px(a, lvl, b, i / a.width, i % a.width, sy, sx);
+    const float sy = (float)a.h[lvl] / (float)H, sx = (float)a.w[lvl] / (float)W;
+    for (int row = 0; row < a.batch * H; ++row)
+      for (int x4 = 0; x4 < W; x4 += 4) {
+        float v[4] = {0.0f, 0.0f, 0.0f, 0.0f};
+        for (int k = 0; k < 4 && x4 + k < W; ++k) v[k] = d2d_forward_px(a, lvl, row / H, row % H, x4 + k, sy, sx);
+        float* o = a.depth + ((size_t)lvl * a.batch * H + row) * W + x4;
+        if (vec) st4g(o, v[0], v[1], v[2], v[3]);
+        else
+          for (int k = 0; k < 4 && x4 + k < W; ++k) o[k] = v[k];
+      }
   }
   return 0;
 }
@@ -322,6 +332,16 @@ static void emu_d2d_fused_level(const bbd_d2d_args& a, int lvl) {
   std::vector<float> srow(a.width);
   for (int b = 0; b < a.batch; ++b)
     for (int iy = 0; iy < a.h[lvl]; ++iy) {
+      if (F == 1) {  // same resolution: four columns per thread, one float4 store (d2d_backward_fused_kernel)
+        const size_t row = (size_t)b * a.h[lvl] + iy;
+        for (int x4 = 0; x4 < a.width; x4 += 4) {
+          float v[4];
+          d2d_fused_col4<1>(a, lvl, b, iy, x4, v);
+          for (int j = 0; j < 4; ++j) v[j] = d2d_epilogue(a, lvl, b, iy, x4 + j, v[j]);
+          st4g(a.gdisp[lvl] + row * a.w[lvl] + x4, v[0], v[1], v[2], v[3]);
+        }
+        continue;
+      }
       for (int x4 = 0; x4 < a.width; x4 += 4) d2d_fused_col4<F>(a, lvl, b, iy, x4, srow.data() + x4);
       for (int ix = 0; ix < a.w[lvl]; ++ix)
         a.gdisp[lvl][((size_t)b * a.h[lvl] + iy) * a.w[lvl] + ix] = d2d_fused_out<F>(a, lvl, b, iy, ix, srow.data());

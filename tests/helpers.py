@@ -142,6 +142,28 @@ def assert_grad_parity(mine, ref32, ref64, key, tol=1e-5, case=None):
     return e
 
 
+def selection_check(win, plan, aux, scales, exact=False):
+    """argmin planes equal the oracle's wherever its best-vs-runner-up margin exceeds 1e-6 (everywhere with
+    ``exact``).  Returns the number of pixels that differ inside the margin."""
+    order = [b for grp in aux["groups"] for b in plan.group_members[grp]]
+    differ = 0
+    for i, s in enumerate(scales):
+        args = torch.cat(aux["argmin"][s], 0)
+        mine = win[i].cpu()[order].long()
+        agree = mine == args
+        if bool(agree.all()):
+            continue
+        assert not exact, (s, int((~agree).sum()))
+        margins = []
+        for p in aux["planes"][s]:
+            top = torch.topk(-p, 2, dim=1).values
+            margins.append(top[:, 0] - top[:, 1])
+        margin = torch.cat(margins, 0)
+        assert bool((agree | (margin <= 1e-6)).all()), (s, int((~agree).sum()))
+        differ += int((~agree).sum())
+    return differ
+
+
 def near_tie_mask(plan, aux, s, dilate=1):
     """(B,H,W) bool: pixels whose best-vs-runner-up margin in the oracle is <= 1e-6, dilated by `dilate`
     pixels (a selection that may legitimately differ changes the gradient of its 3x3 neighbourhood)."""

@@ -10,28 +10,12 @@ import torch
 from baseboostdepth_b200.synthetic import make_batch, make_noise
 from baseboostdepth_b200.trainer import materialise_warps, plan_for
 from fused_util import mirror_to_device, retain_pose_grads, run_fused, to_device
-from helpers import PARITY_LOG, Golden, assert_grad_parity, golden_cases, max_abs, near_tie_mask, pixel_agreement, rel_l2
+from helpers import (PARITY_LOG, Golden, assert_grad_parity, golden_cases, max_abs, near_tie_mask, pixel_agreement, rel_l2,
+                     selection_check)
 from oracle import loss_path as O
 
 pytestmark = pytest.mark.gpu
 CASES = golden_cases()
-
-
-def _selection_check(win, plan, aux, scales, exact=False):
-    """argmin planes equal the oracle's wherever its best-vs-runner-up margin exceeds 1e-6."""
-    order = [b for grp in aux["groups"] for b in plan.group_members[grp]]
-    for i, s in enumerate(scales):
-        args = torch.cat(aux["argmin"][s], 0)
-        mine = win[i].cpu()[order].long()
-        agree = mine == args
-        if bool(agree.all()):
-            continue
-        margins = []
-        for p in aux["planes"][s]:
-            top = torch.topk(-p, 2, dim=1).values
-            margins.append(top[:, 0] - top[:, 1])
-        margin = torch.cat(margins, 0)
-        assert bool((agree | (margin <= 1e-6)).all()), (s, int((~agree).sum()))
 
 
 @pytest.mark.parametrize("case", CASES)
@@ -57,7 +41,7 @@ def test_golden_case_on_gpu(case, cuda_device):
         ref32 = g.params[k].grad if k[0] == "disp" else g.outputs[k].grad
         ref64_ = g64.params[k].grad if k[0] == "disp" else g64.outputs[k].grad
         assert_grad_parity(leaf.grad, ref32, ref64_, k, case=case)
-    _selection_check(ho["argmin"], plan, aux, h.scales, exact=True)
+    selection_check(ho["argmin"], plan, aux, h.scales)
     h.inputs, h.outputs = hi, ho
     with torch.no_grad():
         materialise_warps(h.inputs, h.outputs, h.opt(), plan)
@@ -99,7 +83,7 @@ def test_far_baselines_that_never_win_on_gpu(cuda_device):
     torch.cuda.synchronize()
     for k in ref:
         assert abs(float(losses[k]) - float(ref[k])) <= 2e-6 * max(1.0, abs(float(ref[k]))), k
-    _selection_check(go["argmin"], plan, aux, scales)
+    selection_check(go["argmin"], plan, aux, scales)
     zero_poses = 0
     for k, leaf in leaves.items():
         want = params[k].grad if k[0] == "disp" else outputs[k].grad
@@ -155,7 +139,7 @@ def test_full_size_against_oracle(name, cfg, cuda_device):
         if k[0] == "disp":   # per-pixel: all but the footprints of a few near-ties agree to 1e-4 of the peak
             frac = pixel_agreement(leaf.grad, ref32, tol=1e-4)
             assert frac <= 5e-3 * (1 + k[1]), (k, frac)
-    _selection_check(go["argmin"], plan, aux, scales)
+    selection_check(go["argmin"], plan, aux, scales)
 
 
 # ---- the benchmarked workloads at full size (BASELINE.json configs 2-4, synthetic.WORKLOADS) ----------------
@@ -195,7 +179,7 @@ def test_benched_workload_against_oracle(name, cuda_device):
         ref32 = params[k].grad if k[0] == "disp" else outputs[k].grad
         r64 = p64[k].grad if k[0] == "disp" else o64[k].grad
         assert_grad_parity(leaf.grad, ref32, r64, k, case=name)
-    _selection_check(go["argmin"], plan, aux, scales)
+    selection_check(go["argmin"], plan, aux, scales)
     # per-pixel bar at full resolution
     near = near_tie_mask(plan, aux, 0)
     g_mine, g_ref = leaves[("disp", 0)].grad.cpu()[:, 0].double(), params[("disp", 0)].grad[:, 0].double()
