@@ -675,6 +675,23 @@ static int grid_for(size_t total, int block) {
   return (int)(g < cap ? (g ? g : 1) : cap);
 }
 
+// Sizes of the per-pixel operators, checked before anything is computed from them: a negative count,
+// channel count or size is BBD_E_ARG (it would wrap the size_t element count of a grid-stride loop), a
+// product the kernels form in int (H*W, Ho*Wo, n*channels) that does not fit int32 is BBD_E_RANGE.
+static int check_sizes(const char* who, int64_t n, int64_t channels, int64_t height, int64_t width, int64_t out_h = 0,
+                       int64_t out_w = 0) {
+  static thread_local char msg[128];
+  if (n < 0 || channels < 0 || height < 0 || width < 0 || out_h < 0 || out_w < 0) {
+    snprintf(msg, sizeof(msg), "%s: negative size", who);
+    return fail(BBD_E_ARG, msg);
+  }
+  if (height * width > INT32_MAX || out_h * out_w > INT32_MAX || n * channels > INT32_MAX) {
+    snprintf(msg, sizeof(msg), "%s: size out of the int32 range", who);
+    return fail(BBD_E_RANGE, msg);
+  }
+  return 0;
+}
+
 // ------------------------------------------------------------------------------------------
 // gradients w.r.t. the colour frames (bbd_framegrad.cuh): one thread per pixel, grid-stride
 // ------------------------------------------------------------------------------------------
@@ -1017,7 +1034,8 @@ size_t bbd_d2d_scratch_floats(const bbd_d2d_args* a) {
 int bbd_pose_forward(int32_t n, const float* axisangle, const float* translation, int32_t invert, float* T,
                      bbd_stream_t stream) {
   if (!axisangle || !translation || !T) return fail(BBD_E_ARG, "pose: null argument");
-  if (n <= 0) return 0;
+  if (int rc = check_sizes("pose", n, 1, 1, 1)) return rc;
+  if (n == 0) return 0;
   pose_kernel<<<(n + 63) / 64, 64, 0, (cudaStream_t)stream>>>(n, axisangle, translation, invert, T);
   return check_launch("pose_kernel");
 }
@@ -1025,7 +1043,8 @@ int bbd_pose_forward(int32_t n, const float* axisangle, const float* translation
 int bbd_pose_backward(int32_t n, const float* axisangle, const float* translation, int32_t invert, const float* gT,
                       float* gaxisangle, float* gtranslation, bbd_stream_t stream) {
   if (!axisangle || !translation || !gT || !gaxisangle || !gtranslation) return fail(BBD_E_ARG, "pose backward: null argument");
-  if (n <= 0) return 0;
+  if (int rc = check_sizes("pose backward", n, 1, 1, 1)) return rc;
+  if (n == 0) return 0;
   pose_grad_kernel<<<(n + 63) / 64, 64, 0, (cudaStream_t)stream>>>(n, axisangle, translation, invert, gT, gaxisangle,
                                                                   gtranslation);
   return check_launch("pose_grad_kernel");
@@ -1034,7 +1053,8 @@ int bbd_pose_backward(int32_t n, const float* axisangle, const float* translatio
 int bbd_pose_pack_forward(int32_t n_pose, const float* K, const int32_t* k_row, const float* T, float* P,
                           bbd_stream_t stream) {
   if (!K || !k_row || !T || !P) return fail(BBD_E_ARG, "pose_pack: null argument");
-  if (n_pose <= 0) return 0;
+  if (int rc = check_sizes("pose_pack", n_pose, 12, 1, 1)) return rc;
+  if (n_pose == 0) return 0;
   pose_pack_kernel<<<(n_pose * 12 + 127) / 128, 128, 0, (cudaStream_t)stream>>>(n_pose, K, k_row, T, P);
   return check_launch("pose_pack_kernel");
 }
@@ -1042,7 +1062,8 @@ int bbd_pose_pack_forward(int32_t n_pose, const float* K, const int32_t* k_row, 
 int bbd_pose_pack_backward(int32_t n_pose, const float* K, const int32_t* k_row, const float* gP, float* gT,
                            bbd_stream_t stream) {
   if (!K || !k_row || !gP || !gT) return fail(BBD_E_ARG, "pose_pack backward: null argument");
-  if (n_pose <= 0) return 0;
+  if (int rc = check_sizes("pose_pack backward", n_pose, 16, 1, 1)) return rc;
+  if (n_pose == 0) return 0;
   pose_pack_grad_kernel<<<(n_pose * 16 + 127) / 128, 128, 0, (cudaStream_t)stream>>>(n_pose, K, k_row, gP, gT);
   return check_launch("pose_pack_grad_kernel");
 }
@@ -1050,6 +1071,7 @@ int bbd_pose_pack_backward(int32_t n_pose, const float* K, const int32_t* k_row,
 int bbd_warp_forward(int32_t n, int32_t height, int32_t width, const float* images, const float* depth, const float* inv_K,
                      const float* P, float* warped, float* grid, bbd_stream_t stream) {
   if (!images || !depth || !inv_K || !P || !warped) return fail(BBD_E_ARG, "warp: null argument");
+  if (int rc = check_sizes("warp", n, 3, height, width)) return rc;
   if (n == 0) return 0;
   warp_kernel<<<grid_for((size_t)n * height * width, 256), 256, 0, (cudaStream_t)stream>>>(n, height, width, images, depth,
                                                                                          inv_K, P, warped, grid);
@@ -1059,6 +1081,7 @@ int bbd_warp_forward(int32_t n, int32_t height, int32_t width, const float* imag
 int bbd_backproject_forward(int32_t n, int32_t height, int32_t width, const float* depth, const float* inv_K, float* points,
                             bbd_stream_t stream) {
   if (!depth || !inv_K || !points) return fail(BBD_E_ARG, "backproject: null argument");
+  if (int rc = check_sizes("backproject", n, 4, height, width)) return rc;
   if (n == 0) return 0;
   backproject_kernel<<<grid_for((size_t)n * height * width, 256), 256, 0, (cudaStream_t)stream>>>(n, height, width, depth,
                                                                                                 inv_K, points);
@@ -1068,6 +1091,7 @@ int bbd_backproject_forward(int32_t n, int32_t height, int32_t width, const floa
 int bbd_backproject_backward(int32_t n, int32_t height, int32_t width, const float* inv_K, const float* gpoints,
                              float* gdepth, bbd_stream_t stream) {
   if (!inv_K || !gpoints || !gdepth) return fail(BBD_E_ARG, "backproject backward: null argument");
+  if (int rc = check_sizes("backproject backward", n, 4, height, width)) return rc;
   if (n == 0) return 0;
   backproject_grad_kernel<<<grid_for((size_t)n * height * width, 256), 256, 0, (cudaStream_t)stream>>>(
       n, height, width, inv_K, gpoints, gdepth);
@@ -1077,18 +1101,24 @@ int bbd_backproject_backward(int32_t n, int32_t height, int32_t width, const flo
 int bbd_project_forward(int32_t n, int32_t height, int32_t width, const float* points, const float* P, float eps,
                         float* pix, bbd_stream_t stream) {
   if (!points || !P || !pix) return fail(BBD_E_ARG, "project: null argument");
+  if (int rc = check_sizes("project", n, 4, height, width)) return rc;
   if (n == 0) return 0;
   project_kernel<<<grid_for((size_t)n * height * width, 256), 256, 0, (cudaStream_t)stream>>>(n, height, width, points, P,
                                                                                             eps, pix);
   return check_launch("project_kernel");
 }
 
-int bbd_project_chunks(int32_t height, int32_t width) { return (height * width + PJ_CHUNK - 1) / PJ_CHUNK; }
+int bbd_project_chunks(int32_t height, int32_t width) {
+  if (height <= 0 || width <= 0 || (int64_t)height * width > INT32_MAX) return 0;
+  return (int)(((int64_t)height * width + PJ_CHUNK - 1) / PJ_CHUNK);
+}
 
 int bbd_project_backward(int32_t n, int32_t height, int32_t width, const float* points, const float* P, float eps,
                          const float* gpix, float* gpoints, float* gP_part, bbd_stream_t stream) {
   if (!points || !P || !gpix || !gpoints || !gP_part) return fail(BBD_E_ARG, "project backward: null argument");
-  if (n == 0) return 0;
+  if (int rc = check_sizes("project backward", n, 4, height, width)) return rc;
+  if (n > 65535) return fail(BBD_E_RANGE, "project backward: more than 65535 samples");  // grid.y
+  if (n == 0 || height == 0 || width == 0) return 0;
   dim3 grid(bbd_project_chunks(height, width), n);
   project_grad_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(n, height, width, points, P, eps, gpix, gpoints, gP_part);
   return check_launch("project_grad_kernel");
@@ -1097,6 +1127,7 @@ int bbd_project_backward(int32_t n, int32_t height, int32_t width, const float* 
 int bbd_grid_sample_forward(int32_t n, int32_t channels, int32_t height, int32_t width, int32_t out_h, int32_t out_w,
                             const float* images, const float* grid, float* out, bbd_stream_t stream) {
   if (!images || !grid || !out) return fail(BBD_E_ARG, "grid_sample: null argument");
+  if (int rc = check_sizes("grid_sample", n, channels, height, width, out_h, out_w)) return rc;
   if (n * channels == 0 || out_h * out_w == 0) return 0;
   grid_sample_kernel<<<grid_for((size_t)n * out_h * out_w, 256), 256, 0, (cudaStream_t)stream>>>(
       n, channels, height, width, out_h * out_w, images, grid, out);
@@ -1107,6 +1138,7 @@ int bbd_grid_sample_backward(int32_t n, int32_t channels, int32_t height, int32_
                              const float* images, const float* grid, const float* gout, float* ggrid,
                              bbd_stream_t stream) {
   if (!images || !grid || !gout || !ggrid) return fail(BBD_E_ARG, "grid_sample backward: null argument");
+  if (int rc = check_sizes("grid_sample backward", n, channels, height, width, out_h, out_w)) return rc;
   if (n == 0 || out_h * out_w == 0) return 0;
   grid_sample_grad_kernel<<<grid_for((size_t)n * out_h * out_w, 256), 256, 0, (cudaStream_t)stream>>>(
       n, channels, height, width, out_h * out_w, images, grid, gout, ggrid);
@@ -1132,7 +1164,8 @@ int bbd_loss_combine_backward(int32_t n, const float* g_total, const float* g_pe
 int bbd_project_coords(int32_t n, int32_t height, int32_t width, const float* depth, const float* inv_K, const float* P,
                        float* grid, float* pix, bbd_stream_t stream) {
   if (!depth || !inv_K || !P || (!grid && !pix)) return fail(BBD_E_ARG, "project_coords: null argument");
-  if (n <= 0) return 0;
+  if (int rc = check_sizes("project_coords", n, 2, height, width)) return rc;
+  if (n == 0) return 0;
   stream_coords_kernel<<<grid_for((size_t)n * height * width, 256), 256, 0, (cudaStream_t)stream>>>(n, height, width, depth, inv_K,
                                                                                                    P, grid, pix);
   return check_launch("stream_coords_kernel");
@@ -1141,7 +1174,8 @@ int bbd_project_coords(int32_t n, int32_t height, int32_t width, const float* de
 int bbd_pack_rgba(int32_t n, int32_t height, int32_t width, const float* planar, float* rgba, bbd_stream_t stream) {
   if (!planar || !rgba) return fail(BBD_E_ARG, "pack_rgba: null argument");
   if (!aligned16(rgba)) return fail(BBD_E_ARG, "pack_rgba: rgba must be 16-byte aligned");  // one float4 per pixel
-  if (n <= 0) return 0;
+  if (int rc = check_sizes("pack_rgba", n, 3, height, width)) return rc;
+  if (n == 0) return 0;
   const int HW = height * width;
   const bool vec = (HW % 4 == 0) && aligned16(planar);
   if (vec)
@@ -1168,7 +1202,8 @@ int bbd_u8_to_f32(const uint8_t* src, float* dst, size_t n, bbd_stream_t stream)
 int bbd_grid_sample_dest_keys(int32_t n, int32_t height, int32_t width, int32_t out_h, int32_t out_w, const float* grid,
                               int32_t* keys, bbd_stream_t stream) {
   if (!grid || !keys) return fail(BBD_E_ARG, "grid_sample keys: null argument");
-  if (n <= 0) return 0;
+  if (int rc = check_sizes("grid_sample keys", n, 1, height, width, out_h, out_w)) return rc;
+  if (n == 0) return 0;
   if ((size_t)n * height * width >= (size_t)1 << 31 || (size_t)n * out_h * out_w >= (size_t)1 << 31)
     return fail(BBD_E_RANGE, "grid_sample keys: more than 2^31 elements");
   gs_dest_keys_kernel<<<grid_for((size_t)n * out_h * out_w, 256), 256, 0, (cudaStream_t)stream>>>(n, height, width, out_h * out_w, grid, keys);
@@ -1179,7 +1214,10 @@ int bbd_grid_sample_backward_image(int32_t n, int32_t channels, int32_t height, 
                                    const float* grid, const float* gout, const int32_t* keys_sorted, const int32_t* order,
                                    int32_t* seg_start, float* gimages, bbd_stream_t stream) {
   if (!grid || !gout || !keys_sorted || !order || !seg_start || !gimages) return fail(BBD_E_ARG, "grid_sample image gradient: null argument");
-  if (n <= 0) return 0;
+  if (int rc = check_sizes("grid_sample image gradient", n, channels, height, width, out_h, out_w)) return rc;
+  if (n == 0) return 0;
+  if ((size_t)n * height * width >= (size_t)1 << 31 || (size_t)n * out_h * out_w >= (size_t)1 << 31)
+    return fail(BBD_E_RANGE, "grid_sample image gradient: more than 2^31 elements");
   const int n_items = n * out_h * out_w, n_keys = n * height * width;
   gs_segment_kernel<<<grid_for((size_t)n_items + 1, 256), 256, 0, (cudaStream_t)stream>>>(keys_sorted, n_items, n_keys, seg_start);
   gs_image_grad_kernel<<<grid_for((size_t)n * channels * height * width, 256), 256, 0, (cudaStream_t)stream>>>(
@@ -1190,6 +1228,7 @@ int bbd_grid_sample_backward_image(int32_t n, int32_t channels, int32_t height, 
 int bbd_ssim_forward(int32_t n, int32_t channels, int32_t height, int32_t width, const float* x, const float* y, float* out,
                      bbd_stream_t stream) {
   if (!x || !y || !out) return fail(BBD_E_ARG, "ssim: null argument");
+  if (int rc = check_sizes("ssim", n, channels, height, width)) return rc;
   if (height < 2 || width < 2) return fail(BBD_E_RANGE, "ssim: reflection padding needs at least 2 pixels");
   if (n * channels == 0) return 0;
   ssim_kernel<<<grid_for((size_t)n * channels * height * width, 256), 256, 0, (cudaStream_t)stream>>>(n * channels, height,
@@ -1200,6 +1239,8 @@ int bbd_ssim_forward(int32_t n, int32_t channels, int32_t height, int32_t width,
 int bbd_ssim_backward(int32_t n, int32_t channels, int32_t height, int32_t width, const float* x, const float* y,
                       const float* gout, float* gx, float* gy, bbd_stream_t stream) {
   if (!x || !y || !gout) return fail(BBD_E_ARG, "ssim backward: null argument");
+  if (int rc = check_sizes("ssim backward", n, channels, height, width)) return rc;
+  if (height < 2 || width < 2) return fail(BBD_E_RANGE, "ssim backward: reflection padding needs at least 2 pixels");
   if (n * channels == 0 || (!gx && !gy)) return 0;
   ssim_grad_kernel<<<grid_for((size_t)n * channels * height * width, 128), 128, 0, (cudaStream_t)stream>>>(
       n * channels, height, width, x, y, gout, gx, gy);

@@ -50,7 +50,7 @@ extern "C" {
 #define BBD_MAX_IDENT 6   /* identity candidates per target sample */
 #define BBD_MAX_SCALES 4
 
-#define BBD_E_ARG (-1)   /* null pointer / non-positive size */
+#define BBD_E_ARG (-1)   /* null pointer / negative size (or a size below the stated minimum) */
 #define BBD_E_RANGE (-2) /* table entry or size outside the supported range */
 
 typedef void* bbd_stream_t; /* cudaStream_t */
@@ -289,7 +289,10 @@ int bbd_disp_to_depth_backward_pass2(const bbd_d2d_args* a, int32_t level_begin,
                                      bbd_stream_t stream);
 
 /* ---- module-level operators (tier A: trainer.py unchanged) -----------------
- * Same maths as the layers in layers.py, one kernel each, forward and backward. */
+ * Same maths as the layers in layers.py, one kernel each, forward and backward.
+ * Sizes (here and for bbd_project_coords, bbd_pack_rgba, bbd_pose_* and bbd_pose_pack_*): n == 0 is a
+ * no-op that returns 0 and touches nothing (an empty sub-batch of the trainer reaches these calls); a negative
+ * count, channel count or size is BBD_E_ARG; H*W, Ho*Wo or n*channels above INT32_MAX is BBD_E_RANGE. */
 /* layers.py:160-167; points (n,4,HW) */
 int bbd_backproject_forward(int32_t n, int32_t height, int32_t width, const float* depth,
                             const float* inv_K, float* points, bbd_stream_t stream);
@@ -326,7 +329,7 @@ int bbd_grid_sample_backward_image(int32_t n, int32_t channels, int32_t height, 
                                    int32_t out_w, const float* grid, const float* gout,
                                    const int32_t* keys_sorted, const int32_t* order, int32_t* seg_start,
                                    float* gimages, bbd_stream_t stream);
-/* layers.py:235-249; gx / gy may be NULL */
+/* layers.py:235-249; gx / gy may be NULL; height and width >= 2 (reflection padding), BBD_E_RANGE otherwise */
 int bbd_ssim_forward(int32_t n, int32_t channels, int32_t height, int32_t width, const float* x,
                      const float* y, float* out, bbd_stream_t stream);
 int bbd_ssim_backward(int32_t n, int32_t channels, int32_t height, int32_t width, const float* x,
